@@ -434,6 +434,44 @@ def time_roundtrip(cx: Ctx, rt: RoundTrip, steps: int, warmup: int):
     return total, tp, tu
 
 
+def dump_outputs(rt: RoundTrip, out_dir: str, max_files: int = 1 << 16, max_bytes: int = 1 << 22, seed: int = 7):
+    """Write what the last pack + unpack handed its caller to out_dir/<name>.npy (float32, or float64 where values pass
+    2^24), so that two builds run with the same arguments can be compared array for array.  Per-file arrays keep a seeded
+    sample of at most `max_files` files; the archive and the restored bytes a seeded sample of at most `max_bytes`
+    positions (restored ones inside the files only: the gaps of the output are never written).  At most 44 MB."""
+    torch, dev = rt.cx.torch, rt.cx.dev
+
+    def sample(count, k):
+        return np.sort(np.random.default_rng(seed).choice(count, size=min(count, k), replace=False))
+
+    def take(t, idx):
+        return t[torch.from_numpy(idx.astype(np.int64)).to(dev)].cpu().numpy()
+
+    files = sample(rt.n, max_files)
+    entries = sample(rt.u_n, max_files)
+    nb = int(rt.nbytes[0])
+    arch_pos = np.sort(np.random.default_rng(seed).integers(0, nb, size=min(nb, max_bytes)))
+    lens = rt.mine.len.astype(np.int64)
+    ends = np.cumsum(lens)
+    pos = np.sort(np.random.default_rng(seed).integers(0, rt.B, size=min(rt.B, max_bytes)))
+    f = np.searchsorted(ends, pos, side="right")
+    out_pos = rt.mine.off.astype(np.int64)[f] + pos - (ends[f] - lens[f])
+    arrays = {
+        "pack_digests": take(rt.d_dig[: rt.n * 32].view(rt.n, 32), files).astype(np.float32),
+        "pack_first": take(rt.d_first, files).astype(np.float32),
+        "pack_frame_offset": take(rt.d_foff, files).astype(np.float64),
+        "pack_frame_length": take(rt.d_flen, files).astype(np.float64),
+        "pack_frames_bytes": np.array([nb], dtype=np.float64),
+        "pack_frames_sample": take(rt.d_frames, arch_pos).astype(np.float32),
+        "unpack_ok": take(rt.d_ok, entries).astype(np.float32),
+        "unpack_status": take(rt.d_status, entries).astype(np.float64),
+        "unpack_out_sample": take(rt.d_out, out_pos).astype(np.float32),
+    }
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), a)
+
+
 def leg_roundtrip(cx: Ctx, glob, level: int, steps: int, warmup: int, checksum: bool = True, partition: str = "auto"):
     """One corpus shape, pack + unpack device-resident -> dict for `extras`."""
     rt = RoundTrip(cx, glob, level, checksum=checksum, partition=partition)
@@ -548,12 +586,15 @@ def main():
     ap.add_argument("--cpu-sample-mb-per-core", type=float, default=96.0)
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-e2e", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step returned (a seeded sample) as DIR/<name>.npy")
     args = ap.parse_args()
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
 
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
+    if args.dump_outputs and (args.impl != "ours" or args.config == "c5" or world > 1):
+        ap.error("--dump-outputs needs --impl ours, one GPU and a pack + unpack config (c1-c4)")
     cores = host_cores()
     my_cores = max(1, cores // world)
     args.cpu_cores_used = my_cores * world
@@ -745,6 +786,8 @@ def main():
     launches = lib.zg_kernel_launch_count() - launches0
     lib.zg_profile_enable(0)
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs:
+        dump_outputs(rt, args.dump_outputs)
     tp = sum(x.elapsed_time(y) for x, y in pack_ms) / args.steps
     tu = sum(x.elapsed_time(y) for x, y in unpack_ms) / args.steps
     step_ms = {"pack": [round(x.elapsed_time(y), 2) for x, y in pack_ms], "unpack": [round(x.elapsed_time(y), 2) for x, y in unpack_ms]}
