@@ -995,10 +995,12 @@ k_zds_finish(const u8* __restrict__ archive, const u64* __restrict__ off, const 
 	u32 st = f_status[k];
 	u64 t = tail[k];
 	bool has_ck = (src[4] >> 2) & 1;
+	bool has_fcs = (src[4] >> 5) != 0;  // Frame_Content_Size_Flag or Single_Segment_Flag
 	if (st == ZS_OK && has_ck && t + 4 > len[k]) st = ZS_E_SRC_SIZE;
 	// (Frame_Content_Size, when present, equals ulen for every staged frame: a different total is the corruption the
-	// serial decoder reports at the end of the frame)
-	if (st == ZS_OK && f_out[k] != ulen[k]) st = ZS_E_CORRUPT;
+	// serial decoder reports at the end of the frame.  Without it ulen is only the room there is -- zg_decompress passes
+	// 128 KiB per block -- and the frame may end short of it, as it may on the serial path.)
+	if (st == ZS_OK && has_fcs && f_out[k] != ulen[k]) st = ZS_E_CORRUPT;
 	status[k] = st;
 	produced[k] = st == ZS_OK ? f_out[k] : 0;
 	cksums[2 * (u64)k] = (st == ZS_OK && has_ck) ? zg_ld32(src + t) : 0u;
