@@ -273,12 +273,36 @@ def build_c_oracle(force: bool = False) -> str:
     return so
 
 
+LIT_TYPES = ("raw", "rle", "huf", "treeless")  # Literals_Block_Type 0..3
+SEQ_TABLES = ("ll", "of", "ml")                # in the order of the Symbol_Compression_Modes byte
+SEQ_MODES = ("predefined", "rle", "fse", "repeat")
+NONE_SEEN = (1 << 64) - 1                      # regen_min_*, min_match and huf_min_nw while there was none
+
+
+def lit_header_bytes(st: dict, kind: str) -> dict:
+    """Literals sections of `kind` ("raw", "rle", "huf" or "treeless") per header size in bytes.  Raw / RLE: Size_Format
+    0 and 2 are 1 byte, 1 is 2 bytes, 3 is 3 bytes.  Compressed: Size_Format 0 (1 stream) and 1 (4 streams) are 3 bytes,
+    2 is 4 and 3 is 5."""
+    f = [st[f"lit_{kind}_sf{k}"] for k in range(4)]
+    if kind in ("raw", "rle"):
+        return {1: f[0] + f[2], 2: f[1], 3: f[3]}
+    return {3: f[0] + f[1], 4: f[2], 5: f[3]}
+
+
 class _Stats(ctypes.Structure):
     _fields_ = [
         (n, ctypes.c_uint64)
         for n in (
             "blocks_raw blocks_rle blocks_compressed lit_raw lit_rle lit_huf1 lit_huf4 lit_treeless "
-            "seq_predefined seq_rle seq_fse seq_repeat sequences rep_offsets window_size has_checksum single_segment"
+            "seq_predefined seq_rle seq_fse seq_repeat sequences rep_offsets window_size has_checksum single_segment "
+            + " ".join(f"lit_{t}_sf{f}" for t in LIT_TYPES for f in range(4))
+            + " huf_max_bits huf_wdirect huf_wfse "
+            + " ".join(f"regen_max_{t}" for t in LIT_TYPES) + " "
+            + " ".join(f"regen_min_{t}" for t in LIT_TYPES)
+            + " nseq_h1 nseq_h2 nseq_h3 max_ll_code max_ml_code max_of_code "
+            + " ".join(f"{t}_{m}" for t in SEQ_TABLES for m in SEQ_MODES)
+            + " max_ll_log max_of_log max_ml_log min_match max_match max_offset max_lit_run xblock_matches xblock_reps "
+            "fcs_size blocks huf_max_sym huf_min_nw huf_max_nsym"
         ).split()
     ]
 

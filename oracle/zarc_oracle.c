@@ -270,10 +270,41 @@ static void fse_build(zo_fse_t* t, const int16_t* norm, int nsym, int log) {
 }
 static void fse_build_rle(zo_fse_t* t, uint8_t sym) { t->log = 0; t->e[0].sym = sym; t->e[0].nb = 0; t->e[0].base = 0; }
 
+/* statistics the tests use to make sure every format feature is covered */
+typedef struct {
+	uint64_t blocks_raw, blocks_rle, blocks_compressed;
+	uint64_t lit_raw, lit_rle, lit_huf1, lit_huf4, lit_treeless;
+	uint64_t seq_mode[4]; /* predefined, rle, fse, repeat (summed over LL/OF/ML) */
+	uint64_t sequences, rep_offsets;
+	uint64_t window_size, has_checksum, single_segment;
+	/* ---- coverage of the encoder's edges (what a frame writer chose, not what the input was) ---- */
+	uint64_t lit_fmt[4][4];          /* literals type (raw, rle, huffman, treeless) x Size_Format (0..3) */
+	uint64_t huf_max_bits;           /* largest Huffman max_bits of a tree read */
+	uint64_t huf_wdirect, huf_wfse;  /* Huffman weight descriptions: direct (4-bit) / FSE-compressed */
+	uint64_t regen_max[4], regen_min[4]; /* Regenerated_Size extremes per literals type (min: ~0 while none seen) */
+	uint64_t nseq_hdr[3];            /* Number_of_Sequences fields of 1 / 2 / 3 bytes (nseq = 0 counts as 1 byte) */
+	uint64_t max_ll_code, max_ml_code, max_of_code;
+	uint64_t tab_mode[3][4];         /* table (LL, OF, ML) x mode (predefined, rle, fse, repeat) */
+	uint64_t max_log[3];             /* largest accuracy log of a table built per table (LL, OF, ML; RLE: 0) */
+	uint64_t min_match, max_match;   /* over the resolved sequences (min: ~0 while none seen) */
+	uint64_t max_offset;             /* after repeat codes are resolved */
+	uint64_t max_lit_run;            /* largest Literals_Length of a sequence */
+	uint64_t xblock_matches;         /* matches whose source starts before their block's first output byte */
+	uint64_t xblock_reps;            /* repeat codes that resolve to an offset set in an earlier block */
+	uint64_t fcs_size;               /* Frame_Content_Size field bytes: 0, 1, 2, 4 or 8 */
+	uint64_t blocks;
+	uint64_t huf_max_sym;            /* largest Huffman maxsym (the symbol whose weight is implied) */
+	uint64_t huf_min_nw;             /* fewest explicit weights in a tree description (~0 while none seen) */
+	uint64_t huf_max_nsym;           /* most symbols of non-zero weight in one tree */
+} zo_stats;
+
+#define ZO_MAX(a, b) ((a) = (a) > (uint64_t)(b) ? (a) : (uint64_t)(b))
+#define ZO_MIN(a, b) ((a) = (a) < (uint64_t)(b) ? (a) : (uint64_t)(b))
+
 /* ---- Huffman ---- */
 typedef struct { uint8_t sym[2048]; uint8_t nb[2048]; int max_bits; int valid; } zo_huf_t;
 
-static int huf_read_tree(zo_huf_t* h, const uint8_t* src, size_t n, size_t* used) {
+static int huf_read_tree(zo_huf_t* h, const uint8_t* src, size_t n, size_t* used, zo_stats* st) {
 	uint8_t w[256];
 	int nw = 0, i;
 	uint32_t sum = 0, left;
@@ -334,6 +365,14 @@ static int huf_read_tree(zo_huf_t* h, const uint8_t* src, size_t n, size_t* used
 		}
 	h->max_bits = max_bits;
 	h->valid = 1;
+	if (st) {
+		ZO_MAX(st->huf_max_bits, max_bits);
+		if (src[0] >= 128) st->huf_wdirect++;
+		else st->huf_wfse++;
+		ZO_MAX(st->huf_max_sym, nw - 1);
+		ZO_MIN(st->huf_min_nw, nw - 1);
+		ZO_MAX(st->huf_max_nsym, nw - rank_count[0]);
+	}
 	return 0;
 }
 static int huf_decode_stream(const zo_huf_t* h, const uint8_t* src, size_t n, uint8_t* dst, size_t count) {
@@ -371,22 +410,15 @@ typedef struct {
 	zo_fse_t ll, of, ml;
 	int have_ll, have_of, have_ml;
 	uint64_t rep[3];
+	uint64_t rep_blk[3]; /* block in which each repeat slot's offset was set (the initial 1 / 4 / 8: block 0) */
+	uint64_t blk;        /* index of the block being decoded */
 } zo_frame_state;
 
-/* statistics the tests use to make sure every format feature is covered */
-typedef struct {
-	uint64_t blocks_raw, blocks_rle, blocks_compressed;
-	uint64_t lit_raw, lit_rle, lit_huf1, lit_huf4, lit_treeless;
-	uint64_t seq_mode[4]; /* predefined, rle, fse, repeat (summed over LL/OF/ML) */
-	uint64_t sequences, rep_offsets;
-	uint64_t window_size, has_checksum, single_segment;
-} zo_stats;
-
-static int seq_table(zo_fse_t* t, int* have, int mode, const uint8_t** pp, const uint8_t* end, int max_log, int max_sym,
+static int seq_table(zo_fse_t* t, int* have, int which, int mode, const uint8_t** pp, const uint8_t* end, int max_log, int max_sym,
                      const int16_t* def, int def_n, int def_log, zo_stats* st) {
-	if (st) st->seq_mode[mode]++;
+	if (st) { st->seq_mode[mode]++; st->tab_mode[which][mode]++; }
 	switch (mode) {
-	case 0: fse_build(t, def, def_n, def_log); *have = 1; return 0;
+	case 0: fse_build(t, def, def_n, def_log); *have = 1; if (st) ZO_MAX(st->max_log[which], def_log); return 0;
 	case 1:
 		if (*pp >= end) return -1;
 		if (**pp > max_sym) return -1;
@@ -397,6 +429,7 @@ static int seq_table(zo_fse_t* t, int* have, int mode, const uint8_t** pp, const
 		size_t used;
 		if (fse_read_ncount(*pp, (size_t)(end - *pp), max_log, max_sym, norm, &nsym, &log, &used)) return -1;
 		fse_build(t, norm, nsym, log);
+		if (st) ZO_MAX(st->max_log[which], log);
 		*pp += used; *have = 1; return 0;
 	}
 	default: return *have ? 0 : -1;
@@ -442,7 +475,7 @@ static size_t decode_compressed_block(zo_frame_state* fs, const uint8_t* src, si
 			const uint8_t* lend = p + comp;
 			if (ltype == 2) {
 				size_t used;
-				if (huf_read_tree(&fs->huf, lp, comp, &used)) return ZO_ERR(ZO_E_CORRUPT);
+				if (huf_read_tree(&fs->huf, lp, comp, &used, st)) return ZO_ERR(ZO_E_CORRUPT);
 				lp += used;
 			} else {
 				if (!fs->huf.valid) return ZO_ERR(ZO_E_CORRUPT);
@@ -467,11 +500,18 @@ static size_t decode_compressed_block(zo_frame_state* fs, const uint8_t* src, si
 			p = lend;
 		}
 	}
+	if (st) {
+		st->lit_fmt[ltype][sf]++;
+		ZO_MAX(st->regen_max[ltype], regen);
+		ZO_MIN(st->regen_min[ltype], regen);
+	}
 	/* sequences section */
 	{
 		uint32_t nseq;
 		size_t lpos = 0;
 		if (p >= end) return ZO_ERR(ZO_E_CORRUPT);
+		/* the field length the frame used (a count below 128 may also be written in 2 bytes, one below 0x7F00 in 3) */
+		if (st) st->nseq_hdr[p[0] < 128 ? 0 : p[0] < 255 ? 1 : 2]++;
 		if (p[0] == 0) { nseq = 0; p++; }
 		else if (p[0] < 128) { nseq = p[0]; p++; }
 		else if (p[0] < 255) { if (end - p < 2) return ZO_ERR(ZO_E_CORRUPT); nseq = ((uint32_t)(p[0] - 128) << 8) + p[1]; p += 2; }
@@ -483,9 +523,9 @@ static size_t decode_compressed_block(zo_frame_state* fs, const uint8_t* src, si
 			if (p >= end) return ZO_ERR(ZO_E_CORRUPT);
 			modes = *p++;
 			if (modes & 3) return ZO_ERR(ZO_E_CORRUPT);
-			if (seq_table(&fs->ll, &fs->have_ll, (modes >> 6) & 3, &p, end, 9, 35, LL_DEFAULT, 36, 6, st)) return ZO_ERR(ZO_E_CORRUPT);
-			if (seq_table(&fs->of, &fs->have_of, (modes >> 4) & 3, &p, end, 8, 31, OF_DEFAULT, 29, 5, st)) return ZO_ERR(ZO_E_CORRUPT);
-			if (seq_table(&fs->ml, &fs->have_ml, (modes >> 2) & 3, &p, end, 9, 52, ML_DEFAULT, 53, 6, st)) return ZO_ERR(ZO_E_CORRUPT);
+			if (seq_table(&fs->ll, &fs->have_ll, 0, (modes >> 6) & 3, &p, end, 9, 35, LL_DEFAULT, 36, 6, st)) return ZO_ERR(ZO_E_CORRUPT);
+			if (seq_table(&fs->of, &fs->have_of, 1, (modes >> 4) & 3, &p, end, 8, 31, OF_DEFAULT, 29, 5, st)) return ZO_ERR(ZO_E_CORRUPT);
+			if (seq_table(&fs->ml, &fs->have_ml, 2, (modes >> 2) & 3, &p, end, 9, 52, ML_DEFAULT, 53, 6, st)) return ZO_ERR(ZO_E_CORRUPT);
 			if (bs_init(&b, p, (size_t)(end - p))) return ZO_ERR(ZO_E_CORRUPT);
 			sl = (uint32_t)bs_read(&b, fs->ll.log);
 			so = (uint32_t)bs_read(&b, fs->of.log);
@@ -496,6 +536,7 @@ static size_t decode_compressed_block(zo_frame_state* fs, const uint8_t* src, si
 				uint64_t ov, offset;
 				uint32_t ml, ll;
 				if (oc > 31 || mc > 52 || lc > 35) return ZO_ERR(ZO_E_CORRUPT);
+				if (st) { ZO_MAX(st->max_ll_code, lc); ZO_MAX(st->max_ml_code, mc); ZO_MAX(st->max_of_code, oc); }
 				ov = ((uint64_t)1 << oc) + bs_read(&b, (int)oc);
 				ml = ML_BASE[mc] + (uint32_t)bs_read(&b, ML_BITS[mc]);
 				ll = LL_BASE[lc] + (uint32_t)bs_read(&b, LL_BITS[lc]);
@@ -509,17 +550,25 @@ static size_t decode_compressed_block(zo_frame_state* fs, const uint8_t* src, si
 				if (ov > 3) {
 					offset = ov - 3;
 					fs->rep[2] = fs->rep[1]; fs->rep[1] = fs->rep[0]; fs->rep[0] = offset;
+					fs->rep_blk[2] = fs->rep_blk[1]; fs->rep_blk[1] = fs->rep_blk[0]; fs->rep_blk[0] = fs->blk;
 				} else {
 					uint32_t idx = (uint32_t)ov - 1 + (ll == 0 ? 1 : 0);
+					uint64_t from; /* the block the resolved offset was set in (it keeps that as it moves between slots) */
 					if (st) st->rep_offsets++;
-					if (idx == 0) offset = fs->rep[0];
+					if (idx == 0) { offset = fs->rep[0]; from = fs->rep_blk[0]; }
 					else {
 						offset = idx == 3 ? fs->rep[0] - 1 : fs->rep[idx];
+						from = fs->rep_blk[idx == 3 ? 0 : idx];
 						if (offset == 0) return ZO_ERR(ZO_E_CORRUPT);
-						if (idx > 1) fs->rep[2] = fs->rep[1];
-						fs->rep[1] = fs->rep[0];
-						fs->rep[0] = offset;
+						if (idx > 1) { fs->rep[2] = fs->rep[1]; fs->rep_blk[2] = fs->rep_blk[1]; }
+						fs->rep[1] = fs->rep[0]; fs->rep_blk[1] = fs->rep_blk[0];
+						fs->rep[0] = offset; fs->rep_blk[0] = from;
 					}
+					if (st && from < fs->blk) st->xblock_reps++;
+				}
+				if (st) {
+					ZO_MIN(st->min_match, ml); ZO_MAX(st->max_match, ml);
+					ZO_MAX(st->max_offset, offset); ZO_MAX(st->max_lit_run, ll);
 				}
 				/* execute */
 				if (lpos + ll > regen) return ZO_ERR(ZO_E_CORRUPT);
@@ -527,6 +576,7 @@ static size_t decode_compressed_block(zo_frame_state* fs, const uint8_t* src, si
 				memcpy(dst0 + out, lit + lpos, ll);
 				out += ll; lpos += ll;
 				if (offset > out || offset > window) return ZO_ERR(ZO_E_CORRUPT);
+				if (st && out - offset < dpos) st->xblock_matches++;
 				{
 					uint32_t k;
 					for (k = 0; k < ml; k++) dst0[out + k] = dst0[out + k - offset];
@@ -556,7 +606,12 @@ size_t zo_zstd_decompress_frame(const uint8_t* src, size_t n, uint8_t* dst, size
 	zo_frame_state* fs;
 	uint8_t* litbuf;
 	size_t rc = 0;
-	if (st) memset(st, 0, sizeof *st);
+	if (st) {
+		memset(st, 0, sizeof *st);
+		memset(st->regen_min, 0xff, sizeof st->regen_min);
+		st->min_match = ~(uint64_t)0;
+		st->huf_min_nw = ~(uint64_t)0;
+	}
 	if (n < 6) return ZO_ERR(ZO_E_SRC_SIZE);
 	if (rd32(p) != 0xFD2FB528u) return ZO_ERR(ZO_E_PREFIX);
 	desc = p[4]; p += 5;
@@ -584,7 +639,10 @@ size_t zo_zstd_decompress_frame(const uint8_t* src, size_t n, uint8_t* dst, size
 	if (fcs_len == 2) fcs += 256;
 	p += fcs_len;
 	if (single) window = fcs;
-	if (st) { st->window_size = window; st->has_checksum = (uint64_t)checksum; st->single_segment = (uint64_t)single; }
+	if (st) {
+		st->window_size = window; st->has_checksum = (uint64_t)checksum; st->single_segment = (uint64_t)single;
+		st->fcs_size = (uint64_t)fcs_len;
+	}
 	fs = (zo_frame_state*)calloc(1, sizeof *fs);
 	litbuf = (uint8_t*)malloc(131072 + 32);
 	fs->rep[0] = 1; fs->rep[1] = 4; fs->rep[2] = 8;
@@ -614,6 +672,8 @@ size_t zo_zstd_decompress_frame(const uint8_t* src, size_t n, uint8_t* dst, size
 			out += r; p += bsize;
 			if (st) st->blocks_compressed++;
 		}
+		if (st) st->blocks++;
+		fs->blk++;
 		if (last) break;
 	}
 	if (checksum) {

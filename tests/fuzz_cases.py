@@ -44,7 +44,9 @@ def glued_input(rng, scale=1.0, max_parts=6, sizes=(0, 1, 3, 7, 31, 100, 1000, 5
 
 
 def encode_roundtrips(lib, first, count, levels=(1, 3, 6, 9), log=None):
-    """Frames made by this library's encoder: restored byte-identically by libzstd and by our decoder, digests verified."""
+    """Frames made by this library's encoder: restored byte-identically by libzstd and by our decoder, digests verified;
+    every block independent of the blocks before it (no match reaches into one, no repeat code resolves to an offset set
+    in one: the C oracle's statistics)."""
     frames_done = 0
     for seed in range(first, first + count):
         rng = np.random.default_rng(seed)
@@ -54,6 +56,9 @@ def encode_roundtrips(lib, first, count, levels=(1, 3, 6, 9), log=None):
             for d in datas:
                 fr = bytes(compress2(lib, d, level=level, checksum=bool(rng.integers(0, 2))))
                 assert ref_path.ref_decompress(fr, len(d)) == d, (seed, level, len(d), "libzstd restores something else")
+                got, err, _, st = ref_path.c_zstd_decompress_frame(fr, len(d))
+                assert err == 0 and got == d, (seed, level, len(d), "the C oracle restores something else", err)
+                assert st["xblock_matches"] == 0 and st["xblock_reps"] == 0, (seed, level, len(d), "a block depends on an earlier one")
                 frames.append(fr)
             outs, ok, status, rc = unpack_batch(lib, frames, [len(d) for d in datas], [ref_path.c_blake3(d) for d in datas])
             assert rc == 0 and outs == datas and all(ok), (seed, level, rc, status)

@@ -245,18 +245,23 @@ def test_levels_search_deeper_and_zstd_parameters_are_honoured_or_refused(emu):
     assert _pack_with(emu, files, 3, [(104, 2)])[0] == size[9]
     assert _pack_with(emu, files, 3, [(107, 7)])[0] == size[9]
     assert _pack_with(emu, files, 9, [(107, 1)])[0] == _pack_with(emu, files, 1)[0]  # strategy fast: greedy, one candidate
-    # minMatch: no match shorter than asked for
+    # minMatch: no match shorter than asked for (and tests/test_encoder_edges_emu.py: repeats one byte too short stay
+    # literals)
     from oracle import ref_path as rp
 
     for mm in (5, 7):
         total, frames = _pack_with(emu, files, 3, [(105, mm)])
         assert total > size[3]
-    # windowLog below 16: no offset beyond the window; hashLog: a smaller table finds less
+        for f, fr in zip(files, frames):
+            data, err, consumed, st = rp.c_zstd_decompress_frame(fr, len(f))
+            assert err == 0 and st["sequences"] > 0 and st["min_match"] >= mm, (mm, st["min_match"])
+    # windowLog below 16: no offset beyond the window (and tests/test_encoder_edges_emu.py: a repeat at exactly 2^w is
+    # matched, at 2^w + 1 it is not); hashLog: a smaller table finds less
     total, frames = _pack_with(emu, files, 3, [(101, 10)])
     assert total > size[3]
-    for fr in frames:
-        data, err, consumed, st = rp.c_zstd_decompress_frame(fr, 400_000)
-        assert err == 0 and st["window_size"] >= 0
+    for f, fr in zip(files, frames):
+        data, err, consumed, st = rp.c_zstd_decompress_frame(fr, len(f))
+        assert err == 0 and st["sequences"] > 0 and st["max_offset"] <= 1 << 10, st["max_offset"]
     assert _pack_with(emu, files, 3, [(102, 8)])[0] > size[3]
     assert _pack_with(emu, files, 3, [(102, 20)])[0] == size[3]  # adjusted down to the largest table there is
     # refused: what has no counterpart

@@ -49,20 +49,20 @@ def _into(target: str, make) -> None:
             os.unlink(tmp)
 
 
-def build_product(force: bool = False, verbose: bool = False) -> str:
+def build_product(force: bool = False, verbose: bool = False, target: str = PRODUCT_SO, objdir: str = OBJ, defines=()) -> str:
     """nvcc -> zarc_b200/libzarcgpu.so.  Cross-compiles without a GPU."""
     nvcc = shutil.which("nvcc") or "/usr/local/cuda/bin/nvcc"
-    if not force and not _stale(PRODUCT_SO):
-        return PRODUCT_SO
+    if not force and not _stale(target):
+        return target
     if not os.path.exists(nvcc):
         raise RuntimeError("nvcc not found: cannot build libzarcgpu.so (there is no CPU fallback)")
-    os.makedirs(OBJ, exist_ok=True)
+    os.makedirs(objdir, exist_ok=True)
     objs = []
     procs = []
     for src in _sources():
-        o = os.path.join(OBJ, os.path.basename(src)[:-3] + ".o")
+        o = os.path.join(objdir, os.path.basename(src)[:-3] + ".o")
         objs.append(o)
-        cmd = [nvcc, *NVCC_FLAGS, *os.environ.get("ZG_NVCC_EXTRA", "").split(), "-I", CSRC, "-c", src, "-o", o]
+        cmd = [nvcc, *NVCC_FLAGS, *[f"-D{d}" for d in defines], *os.environ.get("ZG_NVCC_EXTRA", "").split(), "-I", CSRC, "-c", src, "-o", o]
         procs.append((src, subprocess.Popen(cmd, stdout=subprocess.PIPE, stderr=subprocess.STDOUT, text=True)))
     log = []
     for src, p in procs:
@@ -71,28 +71,28 @@ def build_product(force: bool = False, verbose: bool = False) -> str:
         if p.returncode:
             sys.stderr.write(out)
             raise RuntimeError(f"nvcc failed on {src}")
-    with open(os.path.join(OBJ, "ptxas.log"), "w") as f:
+    with open(os.path.join(objdir, "ptxas.log"), "w") as f:
         f.write("\n".join(log))
     if verbose:
         print("\n".join(log))
-    _into(PRODUCT_SO, lambda tmp: subprocess.check_call([nvcc, "-gencode", "arch=compute_100a,code=sm_100a", "-shared", "-o", tmp, *objs, "-lcudart"]))
-    return PRODUCT_SO
+    _into(target, lambda tmp: subprocess.check_call([nvcc, "-gencode", "arch=compute_100a,code=sm_100a", "-shared", "-o", tmp, *objs, "-lcudart"]))
+    return target
 
 
-def build_emu(force: bool = False) -> str:
+def build_emu(force: bool = False, target: str = EMU_SO, objdir: str = os.path.join(OBJ, "emu"), defines=()) -> str:
     """g++ -DZG_EMU -> tests/simt_emu/libzarcgpu_emu.so (TEST INFRASTRUCTURE ONLY)."""
     emu_src = [os.path.join(EMU_DIR, "simt_emu.cpp")]
-    if not force and not _stale(EMU_SO, emu_src + [os.path.join(EMU_DIR, "simt_emu.h")]):
-        return EMU_SO
-    os.makedirs(os.path.join(OBJ, "emu"), exist_ok=True)
+    if not force and not _stale(target, emu_src + [os.path.join(EMU_DIR, "simt_emu.h")]):
+        return target
+    os.makedirs(objdir, exist_ok=True)
     objs = []
     procs = []
     flags = ["-O2", "-g", "-std=c++17", "-fPIC", "-DZG_EMU", "-I", EMU_DIR, "-I", CSRC, "-Wall", "-Wno-unused-function",
              "-Wno-unknown-pragmas", "-Wno-unused-variable", "-Wno-sign-compare", "-Wno-stringop-overflow", "-Wno-maybe-uninitialized", "-Wno-array-bounds"]
     for src in _sources() + emu_src:
-        o = os.path.join(OBJ, "emu", os.path.basename(src).rsplit(".", 1)[0] + ".o")
+        o = os.path.join(objdir, os.path.basename(src).rsplit(".", 1)[0] + ".o")
         objs.append(o)
-        cmd = ["g++", *flags, *os.environ.get("ZG_EMU_EXTRA", "").split(), "-x", "c++", "-c", src, "-o", o]
+        cmd = ["g++", *flags, *[f"-D{d}" for d in defines], *os.environ.get("ZG_EMU_EXTRA", "").split(), "-x", "c++", "-c", src, "-o", o]
         procs.append((src, subprocess.Popen(cmd, stdout=subprocess.PIPE, stderr=subprocess.STDOUT, text=True)))
     for src, p in procs:
         out, _ = p.communicate()
@@ -100,8 +100,29 @@ def build_emu(force: bool = False) -> str:
             sys.stderr.write(out)
         if p.returncode:
             raise RuntimeError(f"g++ (emu) failed on {src}")
-    subprocess.check_call(["g++", "-shared", "-o", EMU_SO, *objs])
-    return EMU_SO
+    _into(target, lambda tmp: subprocess.check_call(["g++", "-shared", "-o", tmp, *objs]))
+    return target
+
+
+# Rare-path builds: the same sources with tuning constants overridden (-DNAME=VALUE), each in its own directory under
+# build/variants/, so that tests can force the paths the defaults take rarely (tests/test_encoder_edges_*.py).  They never
+# touch libzarcgpu.so or libzarcgpu_emu.so.
+VARIANTS = os.path.join(OBJ, "variants")
+
+
+def _variant_dir(defines, kind: str) -> str:
+    name = "_".join(d.replace("=", "-") for d in defines) or "default"
+    return os.path.join(VARIANTS, kind, "".join(c if c.isalnum() or c in "-_" else "_" for c in name))
+
+
+def build_emu_variant(defines, force: bool = False) -> str:
+    d = _variant_dir(defines, "emu")
+    return build_emu(force, target=os.path.join(d, "libzarcgpu_emu.so"), objdir=os.path.join(d, "obj"), defines=defines)
+
+
+def build_product_variant(defines, force: bool = False) -> str:
+    d = _variant_dir(defines, "product")
+    return build_product(force, target=os.path.join(d, "libzarcgpu.so"), objdir=os.path.join(d, "obj"), defines=defines)
 
 
 HOST_DIR = os.path.join(ROOT, "zarc_b200", "host")

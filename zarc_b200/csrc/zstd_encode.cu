@@ -1271,6 +1271,9 @@ ZG_DEV u32 ze_literals_section(ZeWarp* W, const u8* lit, u32 nlit, u8* dst, u32 
 	u32 seg = (nlit + 3) >> 2;
 	u32 comp = 0;
 	if (nlit > 1 && maxc == nlit) {
+		// (not reached by this library's blocks: every byte value of a block is a literal at least once, so literals of one
+		// value come only from a block of one value, and its match finder makes that one literal and one match.  Kept for
+		// any caller that hands over such literals; tests/encoder_edge_cases.py asserts no frame has RLE literals.)
 		mode = 1;
 	} else if (nlit >= 64) {
 		maxbits = ze_huf_build(W, &maxsym);
