@@ -199,7 +199,8 @@ size_t zg_dedup_dev(void* cuda_stream, const uint8_t* digests, uint64_t n, uint8
 /* number of kernels this library has launched in this process (bench.py's gpu_launches) */
 uint64_t zg_kernel_launch_count(void);
 /* optional per-kernel device timing (CUDA events on the launching stream) for roofline reports.
- * k: 0 BLAKE3, 1 Zstd encode, 2 Zstd decode, 3 frame assemble, 4 XXH64, 5 dedup */
+ * k: 0 BLAKE3, 1 Zstd encode, 2 Zstd decode, 3 frame assemble, 4 XXH64, 5 dedup,
+ * 9 Huffman literals decoded ahead of the fused decoder (part of 2) */
 void zg_profile_enable(int on);
 size_t zg_profile_read(int k, double* total_ms, uint64_t* launches);
 

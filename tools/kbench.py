@@ -237,7 +237,7 @@ def main():
         lib.zg_profile_enable(1)
         best, med = timeit(run_unpack, iters=3, warmup=1)
         lib.zg_profile_enable(0)
-        for k, name in ((0, "blake3_verify"), (2, "decode")):
+        for k, name in ((0, "blake3_verify"), (2, "decode"), (9, "huf_literals")):
             ms, cnt = C.c_double(0), C.c_uint64(0)
             lib.zg_profile_read(k, C.byref(ms), C.byref(cnt))
             if cnt.value:

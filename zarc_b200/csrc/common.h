@@ -125,10 +125,14 @@ struct ZgZdWork {
 	ZgBuf queue;    // frame queue counter
 	ZgBuf bins, perm;  // size-sorted hand-out order
 	ZgBuf tiles;       // scan scratch
+	// Huffman literals of the single-block frames, decoded ahead (k_zd_huf_literals): per section its archive offset,
+	// frame, size (then staging offset) and hand-out order; the staged bytes; per frame where its literals are (lit_at)
+	ZgBuf hl_at, hl_frame, hl_off, hl_perm, hl_stage, lit_at;
 	ZgZdStaged st;
 	ZgHostBuf h;
 	void release() {
-		for (ZgBuf* b : {&seqs, &lit, &tabs, &hufsave, &queue, &bins, &perm, &tiles}) b->release();
+		for (ZgBuf* b : {&seqs, &lit, &tabs, &hufsave, &queue, &bins, &perm, &tiles, &hl_at, &hl_frame, &hl_off, &hl_perm, &hl_stage, &lit_at})
+			b->release();
 		st.release();
 		h.release();
 	}
@@ -165,7 +169,7 @@ size_t zg_zstd_encode_run(cudaStream_t s, ZgZeWork& w, const u8* blob, const u64
 // ---- per-kernel device timing (abi.cu): CUDA events on the launching stream, off by default ----
 enum {
 	ZG_K_BLAKE3 = 0, ZG_K_ENCODE = 1 /* the whole encode pass */, ZG_K_DECODE = 2, ZG_K_ASSEMBLE = 3, ZG_K_XXH64 = 4, ZG_K_DEDUP = 5,
-	ZG_K_MATCH = 6, ZG_K_LITERALS = 7, ZG_K_SEQUENCES = 8, ZG_K_COUNT = 9
+	ZG_K_MATCH = 6, ZG_K_LITERALS = 7, ZG_K_SEQUENCES = 8, ZG_K_HUF_LITERALS = 9 /* inside ZG_K_DECODE */, ZG_K_COUNT = 10
 };
 void zg_prof_begin(int k, cudaStream_t s);
 void zg_prof_end(int k, cudaStream_t s);

@@ -74,11 +74,70 @@ __global__ void __launch_bounds__(256) k_zd_bin_scatter(const u64* __restrict__ 
 	if (t < n) perm[atomicAdd(&bins[zd_bin(len[list ? list[t] : t])], 1u)] = (u32)t;
 }
 
+// ---------------------------------------------------------------------------------------------
+// Huffman literals of the single-block frames, decoded ahead of the fused kernel (which then only copies them): in the
+// fused kernel the tree and the streams of a block ran on 1-4 lanes while the rest of the warp waited, frame after frame.
+// Here one warp takes a group of ZD_HL_SECS sections (largest first, so that the streams of a group end together):
+// trees and tables section after section, warp-wide, into the warp's shared memory; then every stream on a lane of its
+// own (lane = 4 x section + stream).  Bytes go to stage + lit_off[s]; lit_at[frame] = lit_off[s], or ZD_LIT_BAD where the
+// fused kernel would have failed the section (bad tree, table, jump table, or a stream that does not end exactly).
+// The trees are read one section after another, so what bounds the kernel is how many sections are in flight per SM:
+// fewer tables per warp hold more warps (B200, 10.2 GB of C2: 8 sections x 2 warps 40.8 ms, 4 x 4 33.4 ms, 2 x 4 23.4 ms,
+// 2 x 2 23.9 ms, 1 x 4 24.5 ms, 1 x 8 24.6 ms).
+#ifndef ZD_HL_SECS
+#define ZD_HL_SECS 2    // sections per warp and group (1..8)
+#endif
+#ifndef ZD_HL_WARPS
+#define ZD_HL_WARPS 4   // warps per CTA
+#endif
+#define ZD_HL_SMEM (sizeof(ZdWarp) + (ZD_HL_SECS - 1) * 2048 * 2)  // per warp: scratch (its table is section 0's) + tables
+ZG_DEV u16* zd_hl_table(ZdWarp* W, u32 i) { return i == 0 ? W->huf : (u16*)(W + 1) + (i - 1) * 2048; }
+
+__global__ void __launch_bounds__(ZD_HL_WARPS * 32)
+k_zd_huf_literals(const u8* __restrict__ archive, const u64* __restrict__ sec_at, const u32* __restrict__ sec_frame,
+                  const u64* __restrict__ lit_off, u64 nsec, const u32* __restrict__ perm, u32* queue, u8* stage, u64* lit_at) {
+	ZG_DYN_SMEM(u8, sm);
+	u32 warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+	ZdWarp* W = (ZdWarp*)(sm + warp * ZD_HL_SMEM);
+	u32 mine = lane >> 2, j = lane & 3;  // my section in the group, my stream in it
+	for (;;) {
+		u32 base = 0;
+		if (lane == 0) base = atomicAdd(queue, (u32)ZD_HL_SECS);
+		base = __shfl_sync(ZG_FULL, base, 0);
+		if (base >= nsec) break;
+		u32 ng = (u32)zg_min<u64>(ZD_HL_SECS, nsec - base);
+		u32 s = 0, bits = 0, sn = 0, first = 0, cnt = 0;
+		const u8* sp = archive;
+		bool has = false, ok = false;
+		for (u32 i = 0; i < ng; i++) {
+			u32 si = perm ? perm[base + i] : base + i;
+			const u8* src = archive + sec_at[si];
+			ZdLitHdr h;
+			zd_lit_header(src, ZS_BLOCK_MAX, h);  // validated by the walk (k_zds_count)
+			const u8* lp = src + h.hdr;
+			u32 nw = 0;
+			u32 used = zd_read_huf_weights(W, lp, h.comp, &nw);
+			u32 hb = used ? zd_build_huf(W, zd_hl_table(W, i), nw) : 0;
+			if (mine == i) {
+				s = si;
+				bits = hb;
+				has = j < h.streams;
+				ok = hb != 0 && zd_huf_split(lp + used, lp + h.comp, h.regen, h.streams, j, sp, sn, first, cnt);
+			}
+		}
+		if (has && ok) ok = zd_huf_stream(zd_hl_table(W, mine), bits, sp, sn, stage + lit_off[s] + first, cnt);
+		u32 bad = __ballot_sync(ZG_FULL, has && !ok);
+		if (mine < ng && j == 0) lit_at[sec_frame[s]] = ((bad >> lane) & 15u) ? ZD_LIT_BAD : lit_off[s];
+		__syncwarp();
+	}
+}
+
 __global__ void __launch_bounds__(ZD_WARPS * 32, ZD_MIN_CTAS)
 k_zstd_decode_frames(const u8* __restrict__ archive, u64 archive_len, const u64* __restrict__ off, const u64* __restrict__ len,
                      const u64* __restrict__ ulen, const u64* __restrict__ out_off, u64 nframes, u8* out, u64 out_cap,
                      const u32* __restrict__ perm, const u32* __restrict__ list, u64* seq_arenas, u8* litbufs, u32* tabs, u8* hufsaves, u32* queue,
-                     u32* status, u64* produced, u32* cksums, u32 cap_div, u32 min_batch, u32 floor_bytes, u32 share_q) {
+                     u32* status, u64* produced, u32* cksums, u32 cap_div, u32 min_batch, u32 floor_bytes, u32 share_q,
+                     const u8* __restrict__ lit_stage, const u64* __restrict__ lit_at) {
 	ZG_DYN_SMEM(ZdWarp, sm);
 	u32 warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
 	ZdWarp* W = &sm[warp];
@@ -152,6 +211,12 @@ k_zstd_decode_frames(const u8* __restrict__ archive, u64 archive_len, const u64*
 				L.cap = ul;
 				L.flags = ZD_F_ACTIVE;
 				zd_frame_header(L);
+				u64 a = lit_at[k];
+				if (a == ZD_LIT_BAD) L.flags |= ZD_F_LIT_BAD;
+				else if (a != ZD_LIT_NONE) {
+					L.flags |= ZD_F_LIT_STAGED;
+					*(const u8**)(hufsave0 + lane * ZD_HUFSAVE + ZD_HUF_STAGED) = lit_stage + a;
+				}
 			}
 		}
 		{
@@ -218,10 +283,45 @@ extern "C" void zg_internal_set_decode_batching(u32 cap_div, u32 min_batch, u32 
 	g_zd_tune[2] = floor_bytes ? floor_bytes : (32u << 10);
 }
 
-// one launch of the fused kernel over `count` frames (those in `list`, or all when it is null), handed out largest first.
+// the nsec sections k_zds_count listed (w.hl_*: nlit bytes in all) -> w.hl_stage, w.lit_at
+static size_t zd_huf_literals_launch(cudaStream_t s, ZgZdWork& w, const u8* archive, u64 nsec, u64 nlit) {
+	if (nsec >= 0xff000000ull) return ZG_ERR(ZG_error_GENERIC);  // (the queue counter runs past nsec by up to one group per warp)
+	if (w.hl_stage.reserve(nlit + 64) || w.hl_perm.reserve(nsec * 4)) return ZG_ERR(ZG_error_memory_allocation);
+	zg_prof_begin(ZG_K_HUF_LITERALS, s);
+	// largest first (the frames' counting sort, over the sizes), then the sizes -> staging offsets
+	u64* sizes = w.hl_off.as<u64>();
+	cudaMemsetAsync(w.bins.p, 0, ZD_BINS * 4, s);
+	u32 g = (u32)((nsec + 255) / 256);
+	ZG_LAUNCH(k_zd_bin_count, g, 256, 0, s, sizes, nullptr, nsec, w.bins.as<u32>());
+	ZG_LAUNCH(k_zd_bin_scan, 1, 1024, 0, s, w.bins.as<u32>());
+	ZG_LAUNCH(k_zd_bin_scatter, g, 256, 0, s, sizes, nullptr, nsec, w.bins.as<u32>(), w.hl_perm.as<u32>());
+	g_zg_launches += 3;
+	size_t r = zg_scan_run(s, w.tiles, sizes, nsec, 0, sizes, nullptr);
+	if (zg_is_error(r)) return r;
+	size_t smem = ZD_HL_SMEM * ZD_HL_WARPS;
+	static ZgPerDevice attr_dev;
+	bool& attr_set = *attr_dev.slot();
+	if (!attr_set) {
+		if (cudaFuncSetAttribute(k_zd_huf_literals, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess)
+			return ZG_ERR(ZG_error_device);
+		attr_set = true;
+	}
+	u64 groups = (nsec + ZD_HL_SECS - 1) / ZD_HL_SECS;
+	u32 per_sm = (u32)zg_max<size_t>(1, (227u << 10) / smem);
+	u32 grid = (u32)zg_min<u64>((groups + ZD_HL_WARPS - 1) / ZD_HL_WARPS, (u64)zg_sm_count() * per_sm);
+	ZG_LAUNCH(k_zd_huf_literals, grid, ZD_HL_WARPS * 32, smem, s, archive, w.hl_at.as<u64>(), w.hl_frame.as<u32>(), sizes, nsec,
+	          w.hl_perm.as<u32>(), w.queue.as<u32>() + 1, w.hl_stage.as<u8>(), w.lit_at.as<u64>());
+	ZG_COUNT_LAUNCH();
+	zg_prof_end(ZG_K_HUF_LITERALS, s);
+	return cudaGetLastError() == cudaSuccess ? 0 : ZG_ERR(ZG_error_device);
+}
+
+// one launch of the fused kernel over `count` frames (those in `list`, or all when it is null), handed out largest first,
+// after the pre-pass over the Huffman literals of the nsec sections k_zds_count listed (nlit bytes).
 // Multi-block frames go through the staged pipeline instead (zstd_decode_staged.cu, which also holds zg_zstd_decode_run).
 size_t zd_fused_launch(cudaStream_t s, ZgZdWork& w, const u8* archive, u64 archive_len, const u64* off, const u64* len, const u64* ulen,
-                       const u64* out_off, const u32* list, u64 count, u8* out, u64 out_cap, u32* status, u64* produced, u32* cksums) {
+                       const u64* out_off, const u32* list, u64 count, u8* out, u64 out_cap, u32* status, u64* produced, u32* cksums,
+                       u64 nsec, u64 nlit) {
 	if (count == 0) return 0;
 	if (count >= 0xff000000ull) return ZG_ERR(ZG_error_GENERIC);  // (the queue counter runs past count by up to one batch per warp)
 	u64 batches = (count + 31) / 32;
@@ -250,9 +350,13 @@ size_t zd_fused_launch(cudaStream_t s, ZgZdWork& w, const u8* archive, u64 archi
 		attr_set = true;
 	}
 	zg_prof_begin(ZG_K_DECODE, s);
+	if (nsec) {
+		size_t r = zd_huf_literals_launch(s, w, archive, nsec, nlit);
+		if (zg_is_error(r)) return r;
+	}
 	ZG_LAUNCH(k_zstd_decode_frames, grid, ZD_WARPS * 32, smem, s, archive, archive_len, off, len, ulen, out_off, count, out, out_cap,
 	          perm, list, w.seqs.as<u64>(), w.lit.as<u8>(), w.tabs.as<u32>(), w.hufsave.as<u8>(), w.queue.as<u32>(), status, produced, cksums,
-	          g_zd_tune[0], g_zd_tune[1], g_zd_tune[2], g_zd_tune[3]);
+	          g_zd_tune[0], g_zd_tune[1], g_zd_tune[2], g_zd_tune[3], w.hl_stage.as<u8>(), w.lit_at.as<u64>());
 	zg_prof_end(ZG_K_DECODE, s);
 	ZG_COUNT_LAUNCH();
 	return cudaGetLastError() == cudaSuccess ? 0 : ZG_ERR(ZG_error_device);

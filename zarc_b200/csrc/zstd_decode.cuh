@@ -38,6 +38,9 @@ struct ZdWarp {
 #define ZD_F_ML_DEF 512u
 #define ZD_F_OF_DEF 1024u
 #define ZD_F_HAS_CK 2048u   // checksum field was read
+#define ZD_F_LIT_STAGED 4096u  // the frame's Huffman literals were decoded ahead (k_zd_huf_literals); where: ZD_HUF_STAGED
+#define ZD_F_LIT_BAD 8192u     // ... and found corrupt
+#define ZD_HUF_STAGED 264u     // offset of that pointer in the lane's Huffman save area (a single-block frame saves no tree)
 
 // one frame's decoding state; lives in the registers of the frame's lane
 struct ZdLane {
@@ -243,8 +246,8 @@ ZG_DEV_NOINLINE u32 zd_read_huf_weights(ZdWarp* W, const u8* src, u32 n, u32* nw
 	return used;
 }
 
-// W->weights[0..nw) -> W->huf.  Returns maxbits (0 on error).  All lanes call.
-ZG_DEV_NOINLINE u32 zd_build_huf(ZdWarp* W, u32 nw) {
+// W->weights[0..nw) -> huf (shared, 1 << maxbits entries).  Returns maxbits (0 on error).  All lanes call.
+ZG_DEV_NOINLINE u32 zd_build_huf(ZdWarp* W, u16* huf, u32 nw) {
 	u32 lane = zg_lane();
 	// weights -> last weight, ranks, per-symbol start index (serial, <= 256 symbols)
 	if (lane == 0) {
@@ -304,13 +307,13 @@ ZG_DEV_NOINLINE u32 zd_build_huf(ZdWarp* W, u32 nw) {
 		u32 start = w ? W->next[s] : 0;
 		u32 entry = s | ((maxbits + 1 - w) << 8);
 		if (len > 0 && len < 32)
-			for (u32 k = 0; k < len; k++) W->huf[start + k] = (u16)entry;
+			for (u32 k = 0; k < len; k++) huf[start + k] = (u16)entry;
 		u32 big = __ballot_sync(ZG_FULL, len >= 32);
 		while (big) {
 			int l = __ffs((int)big) - 1;
 			big &= big - 1;
 			u32 bs = __shfl_sync(ZG_FULL, start, l), bl = __shfl_sync(ZG_FULL, len, l), be = __shfl_sync(ZG_FULL, entry, l);
-			for (u32 k = lane; k < bl; k += 32) W->huf[bs + k] = (u16)be;
+			for (u32 k = lane; k < bl; k += 32) huf[bs + k] = (u16)be;
 		}
 	}
 	__syncwarp();
@@ -345,6 +348,31 @@ ZG_DEV_NOINLINE bool zd_huf_stream(const u16* huf, u32 maxbits, const u8* src, u
 	}
 	zs_back_reload(b);
 	return zs_back_finished(b);
+}
+
+// Where stream j of a Huffman literals section lies: lp..lend = the streams (after the tree description), `streams`
+// 1 or 4 (a 4-stream section starts with its jump table).  Sets the stream's bytes, its first literal and its count
+// (0 streams past the section's count).  Returns false on a bad jump table.
+ZG_DEV bool zd_huf_split(const u8* lp, const u8* lend, u32 regen, u32 streams, u32 j, const u8*& sp, u32& sn, u32& first, u32& cnt) {
+	if (streams == 1) {
+		sp = lp;
+		sn = (u32)(lend - lp);
+		first = 0;
+		cnt = j == 0 ? regen : 0;
+		return true;
+	}
+	if (lend - lp < 10) return false;
+	u32 s1 = zg_ld16(lp), s2 = zg_ld16(lp + 2), s3 = zg_ld16(lp + 4);
+	lp += 6;
+	u32 avail = (u32)(lend - lp);
+	u32 seg = (regen + 3) >> 2;
+	if (s1 + s2 + s3 >= avail || seg * 3 > regen) return false;
+	u32 so = j == 0 ? 0 : j == 1 ? s1 : j == 2 ? s1 + s2 : s1 + s2 + s3;
+	sn = j == 0 ? s1 : j == 1 ? s2 : j == 2 ? s3 : avail - s1 - s2 - s3;
+	sp = lp + so;
+	first = j * seg;
+	cnt = j < 3 ? seg : regen - 3 * seg;
+	return true;
 }
 
 // sequence table for one of LL/OF/ML into the lane's global slot `slot`.  All lanes call (uniform).
@@ -504,6 +532,31 @@ ZG_DEV bool zd_lit_header(const u8* src, u32 n, ZdLitHdr& h) {
 	return h.regen <= ZS_BLOCK_MAX && h.hdr + h.comp <= n && h.regen != 0;
 }
 
+// The literals section of a single-block frame when it is Huffman-coded with a fresh tree (type 2), the only kind
+// k_zd_huf_literals decodes ahead: its archive offset and Regenerated_Size.  Reads the headers exactly as the fused
+// kernel does; anything it cannot take (other literal types, more blocks, bad headers) is left to the fused kernel.
+#define ZD_LIT_NONE (~0ull)        // lit_at[k]: not decoded ahead
+#define ZD_LIT_BAD (~0ull - 1ull)  // ... decoded ahead and corrupt
+ZG_DEV bool zd_single_huf_section(const u8* archive, u64 archive_len, u64 fo, u64 fl, u64& at, u32& regen) {
+	if (fo > archive_len || fl > archive_len - fo) return false;
+	ZdLane L;
+	L.src = archive + fo;
+	L.n = fl;
+	L.status = ZS_OK;
+	L.flags = 0;
+	L.ip = L.fcs = 0;
+	L.fcs_len = 0;
+	zd_frame_header(L);
+	if (L.status != ZS_OK || L.ip + 3 > fl) return false;
+	u32 bh = zg_ld24(L.src + L.ip), bsize = bh >> 3;
+	if ((bh & 7u) != 5u || bsize > ZS_BLOCK_MAX || L.ip + 3 + bsize > fl) return false;  // Last_Block, Compressed_Block
+	ZdLitHdr h;
+	if (!zd_lit_header(L.src + L.ip + 3, bsize, h) || h.ltype != 2) return false;
+	at = fo + L.ip + 3;
+	regen = h.regen;
+	return true;
+}
+
 // The block's literals (uniform in the warp): Raw -> pointer into the block, RLE -> the byte,
 // Huffman -> decoded into litbuf.  Returns a ZS_E_* code.
 ZG_DEV_NOINLINE u32 zd_literals(ZdWarp* W, u32& flags, const u8* src, const ZdLitHdr& h, bool last, u8* litbuf, u8* hufsave, const u8*& lit,
@@ -521,6 +574,12 @@ ZG_DEV_NOINLINE u32 zd_literals(ZdWarp* W, u32& flags, const u8* src, const ZdLi
 		lit = src;
 		return ZS_OK;
 	}
+	if (flags & (ZD_F_LIT_STAGED | ZD_F_LIT_BAD)) {  // a single-block frame's literals, decoded ahead by k_zd_huf_literals
+		if (flags & ZD_F_LIT_BAD) return ZS_E_CORRUPT;
+		flags |= ZD_F_HUF_OK;
+		lit = *(const u8* const*)(hufsave + ZD_HUF_STAGED);
+		return ZS_OK;
+	}
 	const u8* lp = src + h.hdr;
 	const u8* lend = lp + h.comp;
 	u32 regen = h.regen;
@@ -536,7 +595,7 @@ ZG_DEV_NOINLINE u32 zd_literals(ZdWarp* W, u32& flags, const u8* src, const ZdLi
 				hufsave[257] = (u8)(nw >> 8);
 			}
 		}
-		huf_bits = zd_build_huf(W, nw);
+		huf_bits = zd_build_huf(W, W->huf, nw);
 		if (huf_bits == 0) return ZS_E_CORRUPT;
 		flags |= ZD_F_HUF_OK;
 		lp += used;
@@ -546,26 +605,14 @@ ZG_DEV_NOINLINE u32 zd_literals(ZdWarp* W, u32& flags, const u8* src, const ZdLi
 		__syncwarp();
 		for (u32 i = lane; i < nw; i += 32) W->weights[i] = hufsave[i];
 		__syncwarp();
-		huf_bits = zd_build_huf(W, nw);
+		huf_bits = zd_build_huf(W, W->huf, nw);
 		if (huf_bits == 0) return ZS_E_CORRUPT;
 	}
+	const u8* sp;
+	u32 sn, first, cnt;
+	if (!zd_huf_split(lp, lend, regen, h.streams, lane, sp, sn, first, cnt)) return ZS_E_CORRUPT;
 	bool ok = true;
-	if (h.streams == 1) {
-		if (lane == 0) ok = zd_huf_stream(W->huf, huf_bits, lp, (u32)(lend - lp), litbuf, regen);
-	} else {
-		if (lend - lp < 10) return ZS_E_CORRUPT;
-		u32 s1 = zg_ld16(lp), s2 = zg_ld16(lp + 2), s3 = zg_ld16(lp + 4);
-		lp += 6;
-		u32 avail = (u32)(lend - lp);
-		u32 seg = (regen + 3) >> 2;
-		if (s1 + s2 + s3 >= avail || seg * 3 > regen) return ZS_E_CORRUPT;
-		if (lane < 4) {
-			u32 so = lane == 0 ? 0 : lane == 1 ? s1 : lane == 2 ? s1 + s2 : s1 + s2 + s3;
-			u32 sn = lane == 0 ? s1 : lane == 1 ? s2 : lane == 2 ? s3 : avail - s1 - s2 - s3;
-			u32 cnt = lane < 3 ? seg : regen - 3 * seg;
-			ok = zd_huf_stream(W->huf, huf_bits, lp + so, sn, litbuf + lane * seg, cnt);
-		}
-	}
+	if (lane < h.streams) ok = zd_huf_stream(W->huf, huf_bits, sp, sn, litbuf + first, cnt);
 	if (!__all_sync(ZG_FULL, ok)) return ZS_E_CORRUPT;
 	__syncwarp();
 	lit = litbuf;

@@ -118,22 +118,47 @@ ZG_DEV u64 zds_walk(const u8* archive, u64 archive_len, u64 fo, u64 fl, u64 ul, 
 	if (tail) *tail = ip;
 	return nb;
 }
-// tot: [0] staged frames, [1] their blocks, [2] most blocks in one frame, [3] other frames
+// tot: [0] staged frames, [1] their blocks, [2] most blocks in one frame, [3] other frames, [8] Huffman literals sections
+// of single-block frames (decoded ahead by k_zd_huf_literals), [9] their regenerated bytes.  Such a section s is at
+// archive offset sec_at[s] and regenerates sec_len[s] bytes for frame sec_frame[s]; lit_at[k] = ZD_LIT_NONE for the others.
 __global__ void __launch_bounds__(128)
 k_zds_count(const u8* __restrict__ archive, u64 archive_len, const u64* __restrict__ off, const u64* __restrict__ len,
             const u64* __restrict__ ulen, const u64* __restrict__ out_off, u64 out_cap, u64 n, u64 split_min, u32* __restrict__ nblk,
-            u64* __restrict__ first, u32* __restrict__ multi, u32* __restrict__ single, unsigned long long* tot, u32* __restrict__ hist) {
+            u64* __restrict__ first, u32* __restrict__ multi, u32* __restrict__ single, unsigned long long* tot, u32* __restrict__ hist,
+            u64* __restrict__ sec_at, u32* __restrict__ sec_frame, u64* __restrict__ sec_len, u64* __restrict__ lit_at) {
 	u64 k = (u64)blockIdx.x * blockDim.x + threadIdx.x;
-	if (k >= n) return;
-	u64 nb = zds_walk(archive, archive_len, off[k], len[k], ulen[k], out_off[k], out_cap, split_min, (u32)k, nullptr, nullptr);
-	nblk[k] = (u32)nb;
-	if (nb) {
-		multi[atomicAdd(&tot[0], 1ull)] = (u32)k;
-		first[k] = atomicAdd(&tot[1], (unsigned long long)nb);
-		atomicMax(&tot[2], (unsigned long long)nb);
-		atomicAdd(&hist[nb], 1u);
-	} else {
-		single[atomicAdd(&tot[3], 1ull)] = (u32)k;
+	bool sec = false;
+	u64 at = 0;
+	u32 regen = 0;
+	if (k < n) {
+		u64 nb = zds_walk(archive, archive_len, off[k], len[k], ulen[k], out_off[k], out_cap, split_min, (u32)k, nullptr, nullptr);
+		nblk[k] = (u32)nb;
+		if (nb) {
+			multi[atomicAdd(&tot[0], 1ull)] = (u32)k;
+			first[k] = atomicAdd(&tot[1], (unsigned long long)nb);
+			atomicMax(&tot[2], (unsigned long long)nb);
+			atomicAdd(&hist[nb], 1u);
+		} else {
+			single[atomicAdd(&tot[3], 1ull)] = (u32)k;
+			sec = zd_single_huf_section(archive, archive_len, off[k], len[k], at, regen);
+		}
+		if (!sec) lit_at[k] = ZD_LIT_NONE;
+	}
+	// one pair of atomics per warp (about a million sections per 10 GB)
+	u32 m = __ballot_sync(ZG_FULL, sec), lane = zg_lane();
+	if (!m) return;
+	u32 sum = zg_warp_sum(regen);
+	unsigned long long base = 0;
+	if (lane == 0) {
+		base = atomicAdd(&tot[8], (unsigned long long)__popc(m));
+		atomicAdd(&tot[9], (unsigned long long)sum);
+	}
+	base = __shfl_sync(ZG_FULL, base, 0);
+	if (sec) {
+		u64 t = base + (u32)__popc(m & zg_lanemask_lt());
+		sec_at[t] = at;
+		sec_frame[t] = (u32)k;
+		sec_len[t] = regen;
 	}
 }
 __global__ void __launch_bounds__(128)
@@ -315,26 +340,13 @@ ZG_DEV_NOINLINE u32 zds_literals(ZdWarp* W, const u8* src, const ZdLitHdr& h, co
 		if (!tsrc || !zd_lit_header(tsrc, tn, th) || th.ltype != 2) return ZS_E_CORRUPT;
 		if (zd_read_huf_weights(W, tsrc + th.hdr, th.comp, &nw) == 0) return ZS_E_CORRUPT;
 	}
-	huf_bits = zd_build_huf(W, nw);
+	huf_bits = zd_build_huf(W, W->huf, nw);
 	if (huf_bits == 0) return ZS_E_CORRUPT;
-	u32 regen = h.regen;
+	const u8* sp;
+	u32 sn, first, cnt;
+	if (!zd_huf_split(lp, lend, h.regen, h.streams, lane, sp, sn, first, cnt)) return ZS_E_CORRUPT;
 	bool ok = true;
-	if (h.streams == 1) {
-		if (lane == 0) ok = zd_huf_stream(W->huf, huf_bits, lp, (u32)(lend - lp), dst, regen);
-	} else {
-		if (lend - lp < 10) return ZS_E_CORRUPT;
-		u32 s1 = zg_ld16(lp), s2 = zg_ld16(lp + 2), s3 = zg_ld16(lp + 4);
-		lp += 6;
-		u32 avail = (u32)(lend - lp);
-		u32 seg = (regen + 3) >> 2;
-		if (s1 + s2 + s3 >= avail || seg * 3 > regen) return ZS_E_CORRUPT;
-		if (lane < 4) {
-			u32 so = lane == 0 ? 0 : lane == 1 ? s1 : lane == 2 ? s1 + s2 : s1 + s2 + s3;
-			u32 sn = lane == 0 ? s1 : lane == 1 ? s2 : lane == 2 ? s3 : avail - s1 - s2 - s3;
-			u32 cnt = lane < 3 ? seg : regen - 3 * seg;
-			ok = zd_huf_stream(W->huf, huf_bits, lp + so, sn, dst + lane * seg, cnt);
-		}
-	}
+	if (lane < h.streams) ok = zd_huf_stream(W->huf, huf_bits, sp, sn, dst + first, cnt);
 	if (!__all_sync(ZG_FULL, ok)) return ZS_E_CORRUPT;
 	__syncwarp();
 	return ZS_OK;
@@ -1037,7 +1049,8 @@ __global__ void __launch_bounds__(256) k_zds_count_deps(const ZdsBlk* __restrict
 }
 
 size_t zd_fused_launch(cudaStream_t s, ZgZdWork& w, const u8* archive, u64 archive_len, const u64* off, const u64* len, const u64* ulen,
-                       const u64* out_off, const u32* list, u64 count, u8* out, u64 out_cap, u32* status, u64* produced, u32* cksums);
+                       const u64* out_off, const u32* list, u64 count, u8* out, u64 out_cap, u32* status, u64* produced, u32* cksums,
+                       u64 nsec, u64 nlit);
 
 size_t zg_zstd_decode_run(cudaStream_t s, ZgZdWork& w, const u8* archive, u64 archive_len, const u64* off, const u64* len,
                           const u64* ulen, const u64* out_off, u64 n, u8* out, u64 out_cap, u32* status, u64* produced,
@@ -1048,21 +1061,24 @@ size_t zg_zstd_decode_run(cudaStream_t s, ZgZdWork& w, const u8* archive, u64 ar
 	g_zd_stats[0] = g_zd_stats[1] = n;
 	ZgZdStaged& S = w.st;
 	S.xx_n = 0;
-	if (S.nblk.reserve(n * 4) || S.first.reserve(n * 8) || S.multi.reserve(n * 4) || S.single.reserve(n * 4) || S.tot.reserve(64) ||
-	    S.hist.reserve(((size_t)ZDS_HMAX + 2) * 4) || w.h.reserve(64))
+	if (S.nblk.reserve(n * 4) || S.first.reserve(n * 8) || S.multi.reserve(n * 4) || S.single.reserve(n * 4) || S.tot.reserve(128) ||
+	    S.hist.reserve(((size_t)ZDS_HMAX + 2) * 4) || w.h.reserve(128) || w.hl_at.reserve(n * 8) || w.hl_frame.reserve(n * 4) ||
+	    w.hl_off.reserve(n * 8) || w.lit_at.reserve(n * 8))
 		return ZG_ERR(ZG_error_memory_allocation);
-	cudaMemsetAsync(S.tot.p, 0, 64, s);
+	cudaMemsetAsync(S.tot.p, 0, 128, s);
 	cudaMemsetAsync(S.hist.p, 0, ((size_t)ZDS_HMAX + 2) * 4, s);
 	u32 gn = (u32)((n + 127) / 128);
 	unsigned long long* tot = (unsigned long long*)S.tot.p;
 	ZG_LAUNCH(k_zds_count, gn, 128, 0, s, archive, archive_len, off, len, ulen, out_off, out_cap, n, g_zds_split_min, S.nblk.as<u32>(),
-	          S.first.as<u64>(), S.multi.as<u32>(), S.single.as<u32>(), tot, S.hist.as<u32>());
+	          S.first.as<u64>(), S.multi.as<u32>(), S.single.as<u32>(), tot, S.hist.as<u32>(), w.hl_at.as<u64>(), w.hl_frame.as<u32>(),
+	          w.hl_off.as<u64>(), w.lit_at.as<u64>());
 	ZG_COUNT_LAUNCH();
 	u64* h = w.h.as<u64>();
-	if (zg_publish(s, S.tot.p, h, 32) != cudaSuccess || cudaStreamSynchronize(s) != cudaSuccess) return ZG_ERR(ZG_error_device);
-	u64 nmulti = h[0], nblocks = h[1], max_nb = h[2], nsingle = h[3];
+	if (zg_publish(s, S.tot.p, h, 80) != cudaSuccess || cudaStreamSynchronize(s) != cudaSuccess) return ZG_ERR(ZG_error_device);
+	u64 nmulti = h[0], nblocks = h[1], max_nb = h[2], nsingle = h[3], nsec = h[8], nlit = h[9];
 	if (nmulti == 0)  // no multi-block frame: the items are the frames
-		return zd_fused_launch(s, w, archive, archive_len, off, len, ulen, out_off, nullptr, n, out, out_cap, status, produced, cksums);
+		return zd_fused_launch(s, w, archive, archive_len, off, len, ulen, out_off, nullptr, n, out, out_cap, status, produced, cksums, nsec,
+		                       nlit);
 	if (nblocks >= 0xffffffffull) return ZG_ERR(ZG_error_GENERIC);
 	g_zd_stats[1] = nsingle + nblocks;
 	g_zd_stats[3] = nmulti;
@@ -1070,7 +1086,7 @@ size_t zg_zstd_decode_run(cudaStream_t s, ZgZdWork& w, const u8* archive, u64 ar
 	// single-block frames (and whatever the walk refused: the serial decoder names the error) in the fused kernel
 	if (nsingle) {
 		size_t r = zd_fused_launch(s, w, archive, archive_len, off, len, ulen, out_off, S.single.as<u32>(), nsingle, out, out_cap, status,
-		                           produced, cksums);
+		                           produced, cksums, nsec, nlit);
 		if (zg_is_error(r)) return r;
 	}
 	// ---- staged frames ----
