@@ -78,57 +78,119 @@ __global__ void __launch_bounds__(256) k_zd_bin_scatter(const u64* __restrict__ 
 // Huffman literals of the single-block frames, decoded ahead of the fused kernel (which then only copies them): in the
 // fused kernel the tree and the streams of a block ran on 1-4 lanes while the rest of the warp waited, frame after frame.
 // Here one warp takes a group of ZD_HL_SECS sections (largest first, so that the streams of a group end together):
-// trees and tables section after section, warp-wide, into the warp's shared memory; then every stream on a lane of its
-// own (lane = 4 x section + stream).  Bytes go to stage + lit_off[s]; lit_at[frame] = lit_off[s], or ZD_LIT_BAD where the
-// fused kernel would have failed the section (bad tree, table, jump table, or a stream that does not end exactly).
-// The trees are read one section after another, so what bounds the kernel is how many sections are in flight per SM:
-// fewer tables per warp hold more warps (B200, 10.2 GB of C2: 8 sections x 2 warps 40.8 ms, 4 x 4 33.4 ms, 2 x 4 23.4 ms,
-// 2 x 2 23.9 ms, 1 x 4 24.5 ms, 1 x 8 24.6 ms).
+//  1. trees, one lane per section: the lane reads its section's tree description into its own row of weights (FSE-coded
+//     weights through a lane-private table), checks the tree and the jump table, and finds where each weight's entries
+//     start in the table;
+//  2. tables, warp-wide, a round at a time: a round is as many of the next sections as have their tables fit in
+//     ZD_HL_TAB entries (1 << maxbits each) and their streams in 32 lanes.  Each symbol's start in its table is its
+//     weight's start plus the entries of the symbols of that weight before it (match_any over 32 symbols at a time);
+//  3. the round's streams, one per lane (numbered by a prefix over the sections' stream counts).
+// Bytes go to stage + lit_off[s]; lit_at[frame] = lit_off[s], or ZD_LIT_BAD where the fused kernel would have failed the
+// section (bad tree, table, jump table, or a stream that does not end exactly).
+// Tables per round against warps per SM (one CTA per SM; NVIDIA B200 at 1000 W, 10.2 GB of C2, `tools/kbench.py --what
+// pack`, ms of the pre-pass with its sort and scan, all in one call): 16384 entries x 4 warps 21.5 ms, 16384 x 5 18.0,
+// 8192 x 8 12.1 (twice), 6144 x 10 11.5; the warp-wide version before (2 sections x 4 warps, 16 warps per SM) 23.5.
+// 6144 x 10 was measured once, so the defaults stay at 8192 x 8.  More warps per SM is what moved it; which phase
+// bounds it now is not measured.
 #ifndef ZD_HL_SECS
-#define ZD_HL_SECS 2    // sections per warp and group (1..8)
+#define ZD_HL_SECS 32   // sections per warp and group (1..32)
 #endif
 #ifndef ZD_HL_WARPS
-#define ZD_HL_WARPS 4   // warps per CTA
+#define ZD_HL_WARPS 8   // warps per CTA
 #endif
-#define ZD_HL_SMEM (sizeof(ZdWarp) + (ZD_HL_SECS - 1) * 2048 * 2)  // per warp: scratch (its table is section 0's) + tables
-ZG_DEV u16* zd_hl_table(ZdWarp* W, u32 i) { return i == 0 ? W->huf : (u16*)(W + 1) + (i - 1) * 2048; }
+#ifndef ZD_HL_TAB
+#define ZD_HL_TAB 8192  // u16 table entries per warp and round: 4 sections at maxbits 11, more at fewer bits
+#endif
+#define ZD_HL_ROW 284u  // bytes per lane: weights (<= 256 symbols), then u16 start per weight [12]; 71 words, so that
+                        // the lanes' rows start in different banks
+#define ZD_HL_FSE 65u   // u32 per lane of FSE weight table (64 cells), in the table space before the tables are filled
+#define ZD_HL_SMEM (32 * ZD_HL_ROW + 32 + ZD_HL_TAB * 2)  // per warp: rows, stream owners, tables
+static_assert(ZD_HL_SECS >= 1 && ZD_HL_SECS <= 32, "one lane per section");
+static_assert(ZD_HL_TAB >= 2048 && ZD_HL_TAB * 2 >= 32 * ZD_HL_FSE * 4 && ZD_HL_TAB % 8 == 0, "ZD_HL_TAB");
 
 __global__ void __launch_bounds__(ZD_HL_WARPS * 32)
 k_zd_huf_literals(const u8* __restrict__ archive, const u64* __restrict__ sec_at, const u32* __restrict__ sec_frame,
                   const u64* __restrict__ lit_off, u64 nsec, const u32* __restrict__ perm, u32* queue, u8* stage, u64* lit_at) {
 	ZG_DYN_SMEM(u8, sm);
 	u32 warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-	ZdWarp* W = (ZdWarp*)(sm + warp * ZD_HL_SMEM);
-	u32 mine = lane >> 2, j = lane & 3;  // my section in the group, my stream in it
+	u8* rows = sm + warp * ZD_HL_SMEM;
+	u8* owner = rows + 32 * ZD_HL_ROW;        // [32]: the section of each stream lane in the round
+	u16* tabs = (u16*)(owner + 32);           // ZD_HL_TAB entries
+	u8* row = rows + lane * ZD_HL_ROW;
 	for (;;) {
 		u32 base = 0;
 		if (lane == 0) base = atomicAdd(queue, (u32)ZD_HL_SECS);
 		base = __shfl_sync(ZG_FULL, base, 0);
 		if (base >= nsec) break;
 		u32 ng = (u32)zg_min<u64>(ZD_HL_SECS, nsec - base);
-		u32 s = 0, bits = 0, sn = 0, first = 0, cnt = 0;
-		const u8* sp = archive;
-		bool has = false, ok = false;
-		for (u32 i = 0; i < ng; i++) {
-			u32 si = perm ? perm[base + i] : base + i;
+		// 1. my section's tree
+		u32 si = 0, regen = 0, streams = 0, nw = 0, bits = 0;
+		u64 lo = 0;
+		const u8 *lp = archive, *lend = archive;
+		if (lane < ng) {
+			si = perm ? perm[base + lane] : base + lane;
+			lo = lit_off[si];
 			const u8* src = archive + sec_at[si];
 			ZdLitHdr h;
 			zd_lit_header(src, ZS_BLOCK_MAX, h);  // validated by the walk (k_zds_count)
-			const u8* lp = src + h.hdr;
-			u32 nw = 0;
-			u32 used = zd_read_huf_weights(W, lp, h.comp, &nw);
-			u32 hb = used ? zd_build_huf(W, zd_hl_table(W, i), nw) : 0;
-			if (mine == i) {
-				s = si;
-				bits = hb;
-				has = j < h.streams;
-				ok = hb != 0 && zd_huf_split(lp + used, lp + h.comp, h.regen, h.streams, j, sp, sn, first, cnt);
-			}
+			lp = src + h.hdr;
+			lend = lp + h.comp;
+			regen = h.regen;
+			u32 used = zd_read_huf_weights_lane(lp, h.comp, row, (u32*)tabs + lane * ZD_HL_FSE, (u32*)row, &nw);
+			bits = used ? zd_huf_weights_check(row, nw, (u16*)(row + 256)) : 0;
+			lp += used;
+			const u8* sp;
+			u32 sn, first, cnt;
+			if (bits && zd_huf_split(lp, lend, regen, h.streams, 0, sp, sn, first, cnt)) streams = h.streams;
+			else lit_at[sec_frame[si]] = ZD_LIT_BAD;
 		}
-		if (has && ok) ok = zd_huf_stream(zd_hl_table(W, mine), bits, sp, sn, stage + lit_off[s] + first, cnt);
-		u32 bad = __ballot_sync(ZG_FULL, has && !ok);
-		if (mine < ng && j == 0) lit_at[sec_frame[s]] = ((bad >> lane) & 15u) ? ZD_LIT_BAD : lit_off[s];
-		__syncwarp();
+		__syncwarp();  // (the FSE tables are in the space of the Huffman tables)
+		u32 r0 = 0;
+		while (r0 < ng) {
+			// the round: sections r0.. while their tables and streams fit (a section with a bad tree takes neither)
+			u32 mine = lane >= r0 && streams ? (1u << bits) | streams << 20 : 0;
+			u32 incl = zg_warp_incl_scan(mine);
+			u32 r1 = r0 + (u32)__popc(__ballot_sync(ZG_FULL, lane >= r0 && lane < ng && (incl & 0xfffffu) <= ZD_HL_TAB && (incl >> 20) <= 32));
+			bool in = lane >= r0 && lane < r1 && streams;
+			u32 toff = (incl & 0xfffffu) - (mine & 0xfffffu), pre = (incl >> 20) - streams;
+			// 2. tables
+			for (u32 k = r0; k < r1; k++) {
+				u32 kb = __shfl_sync(ZG_FULL, in ? bits : 0, k), knw = __shfl_sync(ZG_FULL, nw, k) + 1, kt = __shfl_sync(ZG_FULL, toff, k);
+				if (!kb) continue;
+				const u8* kw = rows + k * ZD_HL_ROW;
+				u16* rs = (u16*)(kw + 256);  // per weight, where its next symbol's entries start
+				for (u32 s0 = 0; s0 < knw; s0 += 32) {
+					u32 s = s0 + lane, w = s < knw ? kw[s] : 0;
+					u32 peers = __match_any_sync(ZG_FULL, w);
+					u32 start = w ? rs[w] + ((u32)__popc(peers & zg_lanemask_lt()) << (w - 1)) : 0;
+					__syncwarp();
+					if (w && (peers & zg_lanemask_lt()) == 0) rs[w] += (u32)__popc(peers) << (w - 1);
+					zd_huf_fill(tabs + kt, s, w, start, kb);
+					__syncwarp();
+				}
+			}
+			// 3. streams
+			if (in)
+				for (u32 j = 0; j < streams; j++) owner[pre + j] = (u8)lane;
+			__syncwarp();
+			u32 nst = __shfl_sync(ZG_FULL, incl >> 20, r1 - 1);
+			u32 k = lane < nst ? owner[lane] : 0;
+			const u8 *kp = zd_bc(lp, k), *ke = zd_bc(lend, k);
+			u32 kreg = __shfl_sync(ZG_FULL, regen, k), kst = __shfl_sync(ZG_FULL, streams, k), kb = __shfl_sync(ZG_FULL, bits, k);
+			u32 kt = __shfl_sync(ZG_FULL, toff, k), kpre = __shfl_sync(ZG_FULL, pre, k);
+			u64 klo = __shfl_sync(ZG_FULL, lo, k);
+			bool ok = true;
+			if (lane < nst) {
+				const u8* sp;
+				u32 sn, first, cnt;
+				zd_huf_split(kp, ke, kreg, kst, lane - kpre, sp, sn, first, cnt);  // (checked in 1.)
+				ok = zd_huf_stream(tabs + kt, kb, sp, sn, stage + klo + first, cnt);
+			}
+			u32 bad = __ballot_sync(ZG_FULL, !ok);
+			if (in) lit_at[sec_frame[si]] = (bad >> pre) & ((1u << streams) - 1u) ? ZD_LIT_BAD : lo;
+			__syncwarp();
+			r0 = r1;
+		}
 	}
 }
 

@@ -172,26 +172,90 @@ ZG_DEV void zd_warp_match(u8* d, u32 off, u32 ml) {
 }
 
 // ---------------------------------------------------------------------------------------------
+// Huffman tree descriptions (RFC 8878 §4.2.1), read warp-wide (zd_read_huf_weights, zd_build_huf) or one per lane
+// (zd_read_huf_weights_lane, k_zd_huf_literals), both through the single-thread helpers below.
+
+// The description's size from its header byte: direct weights (*nw of them, as nibbles) or FSE-coded (*nw = 0).
+// Returns the bytes it takes (0 when they do not fit in n, or an FSE description is shorter than 2 bytes).
+ZG_DEV u32 zd_huf_desc_size(const u8* src, u32 n, u32* nw) {
+	if (n < 1) return 0;
+	u32 h = src[0];
+	*nw = h >= 128 ? h - 127 : 0;
+	u32 used = h >= 128 ? 1 + ((h - 126) >> 1) : 1 + h;
+	return used > n || h < 2 ? 0 : used;
+}
+ZG_DEV void zd_huf_direct_weights(const u8* src, u32 i, u8* weights) {
+	u32 byte = src[1 + (i >> 1)];
+	weights[i] = (u8)((i & 1) ? (byte & 15) : (byte >> 4));
+}
+// FSE-coded weights after the NCount: two interleaved states; when the stream runs dry after an update, the other
+// state's symbol is the last one (RFC 8878 §4.2.1.2).  Returns how many (0 on error).  Single thread.
+ZG_DEV u32 zd_huf_fse_weights(const u32* tab, u32 log, const u8* src, u32 n, u8* weights) {
+	ZsBack b;
+	if (!zs_back_init(b, src, n)) return 0;
+	u32 cnt = 0;
+	zs_back_reload(b);
+	u32 s1 = zs_back_read(b, log), s2 = zs_back_read(b, log);
+	for (;;) {
+		if (cnt > 253) return 0;
+		u32 e1 = tab[s1];
+		weights[cnt++] = (u8)e1;
+		zs_back_reload(b);
+		s1 = (e1 >> 16) + zs_back_read(b, (e1 >> 8) & 0xff);
+		if (zs_back_overflow(b)) {
+			weights[cnt++] = (u8)tab[s2];
+			return cnt;
+		}
+		u32 e2 = tab[s2];
+		weights[cnt++] = (u8)e2;
+		s2 = (e2 >> 16) + zs_back_read(b, (e2 >> 8) & 0xff);
+		if (zs_back_overflow(b)) {
+			weights[cnt++] = (u8)tab[s1];
+			return cnt;
+		}
+	}
+}
+// The checks of a tree given its explicit weights (all <= 11) as their sum of 2^(w-1) and how many are 1: returns
+// maxbits (0 when the tree is invalid) and sets the implied last weight.
+ZG_DEV u32 zd_huf_tree_check(u32 sum, u32 ones, u32& last) {
+	if (sum == 0) return 0;
+	u32 maxbits = zs_highbit(sum) + 1;
+	u32 left = (1u << maxbits) - sum;
+	if (maxbits > ZS_HUF_MAXLOG || (left & (left - 1))) return 0;
+	last = zs_highbit(left) + 1;
+	ones += last == 1;
+	if (ones < 2 || (ones & 1)) return 0;  // as libzstd HUF_readStats
+	return maxbits;
+}
+// One step of a table fill: the symbol s of weight w (0: none) takes 2^(w-1) entries from `start`.  Short ranges are
+// written by the owning lane, long ones by the warp.  All lanes call.
+ZG_DEV void zd_huf_fill(u16* huf, u32 s, u32 w, u32 start, u32 maxbits) {
+	u32 lane = zg_lane();
+	u32 len = w ? 1u << (w - 1) : 0;
+	u32 entry = s | ((maxbits + 1 - w) << 8);
+	if (len > 0 && len < 32)
+		for (u32 k = 0; k < len; k++) huf[start + k] = (u16)entry;
+	u32 big = __ballot_sync(ZG_FULL, len >= 32);
+	while (big) {
+		int l = __ffs((int)big) - 1;
+		big &= big - 1;
+		u32 bs = __shfl_sync(ZG_FULL, start, l), bl = __shfl_sync(ZG_FULL, len, l), be = __shfl_sync(ZG_FULL, entry, l);
+		for (u32 k = lane; k < bl; k += 32) huf[bs + k] = (u16)be;
+	}
+}
+
 // Huffman tree description -> W->weights[0..nw) (the last weight is implied).  Returns bytes
 // consumed (0 on error).  All lanes call.
 ZG_DEV_NOINLINE u32 zd_read_huf_weights(ZdWarp* W, const u8* src, u32 n, u32* nw_out) {
 	u32 lane = zg_lane();
-	if (n < 1) return 0;
-	u32 h = src[0];
-	u32 used, nw;
-	if (h >= 128) {
-		nw = h - 127;
-		used = 1 + ((nw + 1) >> 1);
-		if (used > n) return 0;
-		for (u32 i = lane; i < nw; i += 32) {
-			u32 byte = src[1 + (i >> 1)];
-			W->weights[i] = (u8)((i & 1) ? (byte & 15) : (byte >> 4));
-		}
+	u32 nw;
+	u32 used = zd_huf_desc_size(src, n, &nw);
+	if (used == 0) return 0;
+	if (nw) {
+		for (u32 i = lane; i < nw; i += 32) zd_huf_direct_weights(src, i, W->weights);
 		__syncwarp();
 	} else {
-		u32 csz = h;
-		used = 1 + csz;
-		if (used > n || csz < 2) return 0;
+		u32 csz = used - 1;
 		if (lane == 0) {
 			u32 nsym = 0, log = 0;
 			u32 nc = zs_read_ncount(src + 1, csz, 6, 255, W->norm, &nsym, &log);
@@ -204,39 +268,7 @@ ZG_DEV_NOINLINE u32 zd_read_huf_weights(ZdWarp* W, const u8* src, u32 n, u32* nw
 		__syncwarp();
 		if (nc == 0 || nc >= csz) return 0;
 		zs_fse_build_dtable(W->tab, W->norm, nsym, log, W->next);
-		if (lane == 0) {
-			ZsBack b;
-			u32 cnt = 0;
-			bool ok = zs_back_init(b, src + 1 + nc, csz - nc);
-			if (ok) {
-				zs_back_reload(b);
-				u32 s1 = zs_back_read(b, log), s2 = zs_back_read(b, log);
-				// two interleaved states; when the stream runs dry after an update, the other
-				// state's symbol is the last one (RFC 8878 §4.2.1.2)
-				for (;;) {
-					if (cnt > 253) {
-						ok = false;
-						break;
-					}
-					u32 e1 = W->tab[s1];
-					W->weights[cnt++] = (u8)e1;
-					zs_back_reload(b);
-					s1 = (e1 >> 16) + zs_back_read(b, (e1 >> 8) & 0xff);
-					if (zs_back_overflow(b)) {
-						W->weights[cnt++] = (u8)W->tab[s2];
-						break;
-					}
-					u32 e2 = W->tab[s2];
-					W->weights[cnt++] = (u8)e2;
-					s2 = (e2 >> 16) + zs_back_read(b, (e2 >> 8) & 0xff);
-					if (zs_back_overflow(b)) {
-						W->weights[cnt++] = (u8)W->tab[s1];
-						break;
-					}
-				}
-			}
-			W->misc[0] = ok ? cnt : 0;
-		}
+		if (lane == 0) W->misc[0] = zd_huf_fse_weights(W->tab, log, src + 1 + nc, csz - nc, W->weights);
 		__syncwarp();
 		nw = W->misc[0];
 		__syncwarp();
@@ -246,12 +278,65 @@ ZG_DEV_NOINLINE u32 zd_read_huf_weights(ZdWarp* W, const u8* src, u32 n, u32* nw
 	return used;
 }
 
+// The same on one lane: the description -> weights[0..nw).  `fse` (64 cells) and `list` (64 words, which may be
+// `weights` itself) are the lane's scratch for FSE-coded weights.
+ZG_DEV u32 zd_read_huf_weights_lane(const u8* src, u32 n, u8* weights, u32* fse, u32* list, u32* nw_out) {
+	u32 nw;
+	u32 used = zd_huf_desc_size(src, n, &nw);
+	if (used == 0) return 0;
+	if (nw) {
+		for (u32 i = 0; i < nw; i++) zd_huf_direct_weights(src, i, weights);
+	} else {
+		u32 csz = used - 1, nsym = 0, log = 0, ne = 0;
+		// the symbols with a nonzero count: at most 1 << log of them (each takes at least one of the cells).  Symbols
+		// above 11 may be declared; a weight above 11 is only an error when it is decoded (zd_huf_tree_check's caller)
+		u32 nc = zs_read_ncount_to(src + 1, csz, 6, 255, [&](u32 s, i32 v) { if (v) list[ne++] = ZS_FSE_ENTRY(s, v); }, &nsym, &log);
+		if (nc == 0 || nc >= csz) return 0;
+		zs_fse_build_dtable_lane(fse, list, ne, log);
+		nw = zd_huf_fse_weights(fse, log, src + 1 + nc, csz - nc, weights);
+		if (nw == 0) return 0;
+	}
+	*nw_out = nw;
+	return used;
+}
+
+// weights[0..nw) -> maxbits (0 when the tree is invalid), the implied last weight at weights[nw], and where each
+// weight's entries start in the table: start[w] for w = 1..11.  Single thread: the counts per weight are kept in
+// registers, as 10-bit fields (three weights per word).
+ZG_DEV u32 zd_huf_weights_check(u8* weights, u32 nw, u16* start) {
+	u32 c0 = 0, c1 = 0, c2 = 0, c3 = 0;
+	bool ok = true;
+	for (u32 i = 0; i < nw; i++) {
+		u32 w = weights[i];
+		ok &= w <= 11;
+		u32 q = (w * 11) >> 5, inc = w <= 11 ? 1u << ((w - 3 * q) * 10) : 0;  // (q = w / 3 for w <= 11)
+		c0 += q == 0 ? inc : 0;
+		c1 += q == 1 ? inc : 0;
+		c2 += q == 2 ? inc : 0;
+		c3 += q == 3 ? inc : 0;
+	}
+	auto count = [&](u32 w) { return ((w < 3 ? c0 : w < 6 ? c1 : w < 9 ? c2 : c3) >> ((w % 3) * 10)) & 1023u; };
+	u32 sum = 0, last = 0;
+	ZG_UNROLL
+	for (u32 w = 1; w <= 11; w++) sum += count(w) << (w - 1);
+	u32 maxbits = ok ? zd_huf_tree_check(sum, count(1), last) : 0;
+	if (maxbits == 0) return 0;
+	weights[nw] = (u8)last;
+	u32 at = 0;
+	ZG_UNROLL
+	for (u32 w = 1; w <= 11; w++) {
+		start[w] = (u16)at;
+		at += (count(w) + (w == last)) << (w - 1);
+	}
+	return maxbits;
+}
+
 // W->weights[0..nw) -> huf (shared, 1 << maxbits entries).  Returns maxbits (0 on error).  All lanes call.
 ZG_DEV_NOINLINE u32 zd_build_huf(ZdWarp* W, u16* huf, u32 nw) {
 	u32 lane = zg_lane();
 	// weights -> last weight, ranks, per-symbol start index (serial, <= 256 symbols)
 	if (lane == 0) {
-		u32 sum = 0;
+		u32 sum = 0, maxbits = 0, last = 0;
 		bool ok = true;
 		u32 rank[13];
 		for (u32 i = 0; i < 13; i++) rank[i] = 0;
@@ -263,19 +348,11 @@ ZG_DEV_NOINLINE u32 zd_build_huf(ZdWarp* W, u16* huf, u32 nw) {
 				rank[w]++;
 			}
 		}
-		u32 maxbits = 0;
-		if (ok && sum != 0) {
-			maxbits = zs_highbit(sum) + 1;
-			u32 left = (1u << maxbits) - sum;
-			if (maxbits > ZS_HUF_MAXLOG || (left & (left - 1))) ok = false;
-			else {
-				u32 last = zs_highbit(left) + 1;
-				W->weights[nw] = (u8)last;
-				rank[last]++;
-			}
-		} else ok = false;
-		if (ok && (rank[1] < 2 || (rank[1] & 1))) ok = false;  // as libzstd HUF_readStats
+		if (ok) maxbits = zd_huf_tree_check(sum, rank[1], last);
+		ok = maxbits != 0;
 		if (ok) {
+			W->weights[nw] = (u8)last;
+			rank[last]++;
 			u32 start = 0;
 			u32 rs[13];
 			for (u32 w = 1; w <= 11; w++) {
@@ -299,50 +376,44 @@ ZG_DEV_NOINLINE u32 zd_build_huf(ZdWarp* W, u16* huf, u32 nw) {
 	__syncwarp();
 	if (!ok) return 0;
 	nw += 1;
-	// fill: long ranges cooperatively, short ranges by the owning lane
 	for (u32 s0 = 0; s0 < nw; s0 += 32) {
 		u32 s = s0 + lane;
 		u32 w = s < nw ? W->weights[s] : 0;
-		u32 len = w ? 1u << (w - 1) : 0;
-		u32 start = w ? W->next[s] : 0;
-		u32 entry = s | ((maxbits + 1 - w) << 8);
-		if (len > 0 && len < 32)
-			for (u32 k = 0; k < len; k++) huf[start + k] = (u16)entry;
-		u32 big = __ballot_sync(ZG_FULL, len >= 32);
-		while (big) {
-			int l = __ffs((int)big) - 1;
-			big &= big - 1;
-			u32 bs = __shfl_sync(ZG_FULL, start, l), bl = __shfl_sync(ZG_FULL, len, l), be = __shfl_sync(ZG_FULL, entry, l);
-			for (u32 k = lane; k < bl; k += 32) huf[bs + k] = (u16)be;
-		}
+		zd_huf_fill(huf, s, w, w ? W->next[s] : 0, maxbits);
 	}
 	__syncwarp();
 	return maxbits;
 }
 
-// one Huffman stream, single thread
+// one Huffman stream, single thread.  Four symbols per refill of the bit container, stored as one aligned word (byte
+// stores up to the first 4-byte boundary of dst and at the end): lanes decoding different streams write to different
+// lines, so every store instruction costs the memory system one request per lane.
 ZG_DEV_NOINLINE bool zd_huf_stream(const u16* huf, u32 maxbits, const u8* src, u32 n, u8* dst, u32 count) {
 	ZsBack b;
 	if (!zs_back_init(b, src, n)) return false;
 	u32 i = 0;
 	const u32 sh = 32u - maxbits;
+	const u32 head = zg_min<u32>(count, (u32)(0u - (uintptr_t)dst) & 3u);
 	while (i < count) {
 		zs_back_reload(b);
-		u32 m = zg_min<u32>(count - i, 5u);  // 5 x 11 bits <= 57
+		u32 m = i < head ? head - i : zg_min<u32>(count - i, 4u);  // 4 x 11 bits <= 57
 		// the unread bits left-aligned in ah:al; every symbol then costs one shift for the index and a two-word
 		// shift for the bits it used (bits before the start of the stream shift in as zeros)
 		u32 c = b.consumed;
 		u32 ah = c < 32 ? __funnelshift_l(b.lo, b.hi, c) : (c < 64 ? b.lo << (c & 31u) : 0u);
 		u32 al = c < 32 ? b.lo << c : 0u;
-		u32 used = 0;
+		u32 used = 0, word = 0;
 		for (u32 k = 0; k < m; k++) {
 			u32 e = huf[ah >> sh];
-			dst[i + k] = (u8)e;
+			word |= (e & 0xffu) << (8 * k);
 			u32 nb = e >> 8;
 			ah = __funnelshift_l(al, ah, nb);
 			al <<= nb;
 			used += nb;
 		}
+		if (m == 4) *(u32*)(dst + i) = word;
+		else
+			for (u32 k = 0; k < m; k++) dst[i + k] = (u8)(word >> (8 * k));
 		b.consumed = c + used;
 		i += m;
 	}
