@@ -2,8 +2,8 @@
 per tree), with tree descriptions, jump tables and streams at every edge it checks.  They run in batches of more than
 32 frames, good and bad shuffled together, so that a bad tree shares a warp's group of sections with good ones.  Every
 verdict is checked three ways: against the case's expected verdict, against libzstd, and against the same literals in
-a two-block frame, which the decoder reads through its warp-wide tree path instead.  Shared by
-tests/test_huf_trees_emu.py and tests/test_huf_trees_gpu.py."""
+a two-block frame, which is not decoded ahead: the warp that decodes its block reads the tree there, on whichever path
+takes the frame.  Shared by tests/test_huf_trees_emu.py and tests/test_huf_trees_gpu.py."""
 import struct
 
 import numpy as np

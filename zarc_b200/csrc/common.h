@@ -121,7 +121,7 @@ struct ZgZdWork {
 	ZgBuf seqs;     // per-warp sequence arenas
 	ZgBuf lit;      // per-warp literal buffers
 	ZgBuf tabs;     // per-lane FSE decode-table slots
-	ZgBuf hufsave;  // per-lane Huffman weights (Treeless blocks)
+	ZgBuf hufsave;  // per-lane ZdHufSave: where the last Huffman tree description (Treeless blocks) and staged literals are
 	ZgBuf queue;    // frame queue counter
 	ZgBuf bins, perm;  // size-sorted hand-out order
 	ZgBuf tiles;       // scan scratch

@@ -19,8 +19,9 @@
 //      literals, its sequences and its recent output (the match sources) are cache-hot.
 // Blocks of a frame stay in order, so Treeless literals, Repeat_Mode tables, repeat offsets and
 // cross-block matches (all produced by libzstd at levels 1/3/9, SURVEY.md App. E) work.  State that
-// must outlive a round lives in global scratch: the FSE tables (fixed slot per lane) and the Huffman
-// weights (for Treeless blocks).  A block whose sequences do not fit the arena waits for the next round.
+// must outlive a round lives in global scratch: the FSE tables (fixed slot per lane) and where the
+// last Huffman tree description is (Treeless blocks read it again).  A block whose sequences do not fit
+// the arena waits for the next round.
 // HBM traffic: C read + N written (+ 8 B per sequence and the literals staged through L2).
 //
 // This kernel takes the single-block frames (every file up to 128 KiB: almost all of a source tree) and whatever the
@@ -157,17 +158,8 @@ k_zd_huf_literals(const u8* __restrict__ archive, const u64* __restrict__ sec_at
 			for (u32 k = r0; k < r1; k++) {
 				u32 kb = __shfl_sync(ZG_FULL, in ? bits : 0, k), knw = __shfl_sync(ZG_FULL, nw, k) + 1, kt = __shfl_sync(ZG_FULL, toff, k);
 				if (!kb) continue;
-				const u8* kw = rows + k * ZD_HL_ROW;
-				u16* rs = (u16*)(kw + 256);  // per weight, where its next symbol's entries start
-				for (u32 s0 = 0; s0 < knw; s0 += 32) {
-					u32 s = s0 + lane, w = s < knw ? kw[s] : 0;
-					u32 peers = __match_any_sync(ZG_FULL, w);
-					u32 start = w ? rs[w] + ((u32)__popc(peers & zg_lanemask_lt()) << (w - 1)) : 0;
-					__syncwarp();
-					if (w && (peers & zg_lanemask_lt()) == 0) rs[w] += (u32)__popc(peers) << (w - 1);
-					zd_huf_fill(tabs + kt, s, w, start, kb);
-					__syncwarp();
-				}
+				u8* kw = rows + k * ZD_HL_ROW;
+				zd_huf_fill_table(tabs + kt, kw, knw, (u16*)(kw + 256), kb);
 			}
 			// 3. streams
 			if (in)
@@ -197,7 +189,7 @@ k_zd_huf_literals(const u8* __restrict__ archive, const u64* __restrict__ sec_at
 __global__ void __launch_bounds__(ZD_WARPS * 32, ZD_MIN_CTAS)
 k_zstd_decode_frames(const u8* __restrict__ archive, u64 archive_len, const u64* __restrict__ off, const u64* __restrict__ len,
                      const u64* __restrict__ ulen, const u64* __restrict__ out_off, u64 nframes, u8* out, u64 out_cap,
-                     const u32* __restrict__ perm, const u32* __restrict__ list, u64* seq_arenas, u8* litbufs, u32* tabs, u8* hufsaves, u32* queue,
+                     const u32* __restrict__ perm, const u32* __restrict__ list, u64* seq_arenas, u8* litbufs, u32* tabs, ZdHufSave* hufsaves, u32* queue,
                      u32* status, u64* produced, u32* cksums, u32 cap_div, u32 min_batch, u32 floor_bytes, u32 share_q,
                      const u8* __restrict__ lit_stage, const u64* __restrict__ lit_at) {
 	ZG_DYN_SMEM(ZdWarp, sm);
@@ -207,7 +199,7 @@ k_zstd_decode_frames(const u8* __restrict__ archive, u64 archive_len, const u64*
 	u64* arena = seq_arenas + gw * ZD_SEQ_ARENA;
 	u8* litbuf = litbufs + gw * ZD_LITBUF;
 	u32* my_slot = tabs + (gw * 32 + lane) * ZD_TAB_SLOT;
-	u8* hufsave0 = hufsaves + gw * 32 * ZD_HUFSAVE;
+	ZdHufSave* hufsave = hufsaves + gw * 32;
 	u64 hint_len = ~0ull;  // compressed size of the last item of this warp's previous batch
 	u64 prev_base = 0;
 	for (;;) {
@@ -251,15 +243,15 @@ k_zstd_decode_frames(const u8* __restrict__ archive, u64 archive_len, const u64*
 		L.status = ZS_OK;
 		L.flags = 0;
 		L.fcs_len = L.cksum = 0;
-		L.rep0 = 1;
-		L.rep1 = 4;
-		L.rep2 = 8;
+		L.seq.rep0 = 1;
+		L.seq.rep1 = 4;
+		L.seq.rep2 = 8;
 		L.ll_log = L.ml_log = L.of_log = 0;
 		L.blk = archive;
-		L.blk_n = L.nseq = L.nseq_left = L.seq_base = 0;
-		L.b.start = L.b.ptr = archive;
-		L.b.lo = L.b.hi = L.b.consumed = 0;
-		L.sl = L.so = L.sm = 0;
+		L.blk_n = L.nseq = L.seq.left = L.seq_base = 0;
+		L.seq.b.start = L.seq.b.ptr = archive;
+		L.seq.b.lo = L.seq.b.hi = L.seq.b.consumed = 0;
+		L.seq.sl = L.seq.so = L.seq.sm = 0;
 		u64 mylen = 0;
 		if (mine) {
 			u64 fo = off[k], fl = len[k], ul = ulen[k], oo = out_off[k];
@@ -272,12 +264,20 @@ k_zstd_decode_frames(const u8* __restrict__ archive, u64 archive_len, const u64*
 				L.out = out + oo;
 				L.cap = ul;
 				L.flags = ZD_F_ACTIVE;
-				zd_frame_header(L);
+				ZdFrameHdr F;
+				u32 st = zd_frame_header(L.src, L.n, F);
+				if (st != ZS_OK) zd_fail(L, st);
+				else {
+					L.ip = F.ip;
+					L.fcs = F.fcs;
+					L.fcs_len = F.fcs_len;
+					if (F.cksum) L.flags |= ZD_F_CKSUM;
+				}
 				u64 a = lit_at[k];
 				if (a == ZD_LIT_BAD) L.flags |= ZD_F_LIT_BAD;
 				else if (a != ZD_LIT_NONE) {
 					L.flags |= ZD_F_LIT_STAGED;
-					*(const u8**)(hufsave0 + lane * ZD_HUFSAVE + ZD_HUF_STAGED) = lit_stage + a;
+					hufsave[lane].staged = lit_stage + a;
 				}
 			}
 		}
@@ -297,7 +297,7 @@ k_zstd_decode_frames(const u8* __restrict__ archive, u64 archive_len, const u64*
 				int f = __ffs((int)todo) - 1;
 				todo &= todo - 1;
 				ZdLane U = zd_bcast(L, f);
-				zd_setup_frame(W, U, tabs + (gw * 32 + (u32)f) * ZD_TAB_SLOT, arena_used, litbuf, hufsave0 + (u32)f * ZD_HUFSAVE);
+				zd_setup_frame(W, U, tabs + (gw * 32 + (u32)f) * ZD_TAB_SLOT, arena_used, litbuf, hufsave + f);
 				if (lane == (u32)f) L = U;
 				__syncwarp();
 			}
@@ -306,10 +306,11 @@ k_zstd_decode_frames(const u8* __restrict__ archive, u64 archive_len, const u64*
 				const u32* llt = (L.flags & ZD_F_LL_DEF) ? ZS_LL_DEFAULT_DTABLE : my_slot;
 				const u32* mlt = (L.flags & ZD_F_ML_DEF) ? ZS_ML_DEFAULT_DTABLE : my_slot + 512;
 				const u32* oft = (L.flags & ZD_F_OF_DEF) ? ZS_OF_DEFAULT_DTABLE : my_slot + 1024;
+				ZdSeqPlain plain;
 				for (;;) {
-					u32 cnt = zg_min<u32>((u32)ZD_B_STEPS, L.nseq_left);
+					u32 cnt = zg_min<u32>((u32)ZD_B_STEPS, L.seq.left);
 					if (!__any_sync(ZG_FULL, cnt > 0)) break;
-					if (cnt && !zd_lane_decode(L, cnt, llt, mlt, oft, arena + L.seq_base + (L.nseq - L.nseq_left))) zd_fail(L, ZS_E_CORRUPT);
+					if (cnt && !zd_lane_decode(L.seq, plain, cnt, llt, mlt, oft, arena + L.seq_base + (L.nseq - L.seq.left))) zd_fail(L, ZS_E_CORRUPT);
 				}
 			}
 			__syncwarp();
@@ -319,7 +320,7 @@ k_zstd_decode_frames(const u8* __restrict__ archive, u64 archive_len, const u64*
 				int f = __ffs((int)todo) - 1;
 				todo &= todo - 1;
 				ZdLane U = zd_bcast(L, f);
-				zd_exec_block(W, U, arena + U.seq_base, litbuf, hufsave0 + (u32)f * ZD_HUFSAVE);
+				zd_exec_block(W, U, arena + U.seq_base, litbuf, hufsave + f);
 				if (lane == (u32)f) L = U;
 				__syncwarp();
 			}
@@ -390,7 +391,7 @@ size_t zd_fused_launch(cudaStream_t s, ZgZdWork& w, const u8* archive, u64 archi
 	u32 grid = (u32)zg_min<u64>((batches + ZD_WARPS - 1) / ZD_WARPS, (u64)zg_sm_count() * ZD_MIN_CTAS);
 	size_t warps = (size_t)grid * ZD_WARPS;
 	if (w.seqs.reserve(warps * ZD_SEQ_ARENA * 8) || w.lit.reserve(warps * ZD_LITBUF) || w.tabs.reserve(warps * 32 * ZD_TAB_SLOT * 4) ||
-	    w.hufsave.reserve(warps * 32 * ZD_HUFSAVE) || w.queue.reserve(16) || w.bins.reserve(ZD_BINS * 4) || w.perm.reserve(count * 4))
+	    w.hufsave.reserve(warps * 32 * sizeof(ZdHufSave)) || w.queue.reserve(16) || w.bins.reserve(ZD_BINS * 4) || w.perm.reserve(count * 4))
 		return ZG_ERR(ZG_error_memory_allocation);
 	cudaMemsetAsync(w.queue.p, 0, 16, s);
 	const u32* perm = nullptr;
@@ -417,7 +418,7 @@ size_t zd_fused_launch(cudaStream_t s, ZgZdWork& w, const u8* archive, u64 archi
 		if (zg_is_error(r)) return r;
 	}
 	ZG_LAUNCH(k_zstd_decode_frames, grid, ZD_WARPS * 32, smem, s, archive, archive_len, off, len, ulen, out_off, count, out, out_cap,
-	          perm, list, w.seqs.as<u64>(), w.lit.as<u8>(), w.tabs.as<u32>(), w.hufsave.as<u8>(), w.queue.as<u32>(), status, produced, cksums,
+	          perm, list, w.seqs.as<u64>(), w.lit.as<u8>(), w.tabs.as<u32>(), w.hufsave.as<ZdHufSave>(), w.queue.as<u32>(), status, produced, cksums,
 	          g_zd_tune[0], g_zd_tune[1], g_zd_tune[2], g_zd_tune[3], w.hl_stage.as<u8>(), w.lit_at.as<u64>());
 	zg_prof_end(ZG_K_DECODE, s);
 	ZG_COUNT_LAUNCH();

@@ -13,16 +13,15 @@
 #define ZD_SEQ_ARENA (1u << 17)          // u64 entries of sequence staging per warp (1 MiB)
 #define ZD_LITBUF (ZS_BLOCK_MAX + 64)    // bytes of literal staging per warp
 #define ZD_TAB_SLOT 1280u                // u32 entries per lane: LL 512 | ML 512 | OF 256
-#define ZD_HUFSAVE 272u                  // bytes per lane: 256 weights + count
 #define ZD_OFF_MAX ((1u << 28) - 1u)
 #define ZD_BATCH_BYTES (128u << 10)        // least compressed bytes per warp batch (see the hand-out in the kernel)
 
 struct ZdWarp {
 	u32 tab[512];      // table under construction (FSE sequence table or Huffman-weight table)
 	u16 huf[2048];     // sym | nbBits << 8
-	u8 weights[256];
+	u8 weights[256];   // Huffman weights (and, while FSE-coded ones are read, the list of nonzero counts)
 	i16 norm[256];
-	u16 next[256];
+	u16 next[256];     // FSE build scratch; Huffman: where each weight's table entries start
 	u32 misc[8];
 };
 
@@ -30,7 +29,7 @@ struct ZdWarp {
 #define ZD_F_ACTIVE 1u      // frame still has blocks to decode
 #define ZD_F_LAST 2u        // the block in flight is the frame's last
 #define ZD_F_CKSUM 4u       // frame has a Content_Checksum
-#define ZD_F_HUF_OK 8u      // a Huffman table has been defined (saved weights are valid)
+#define ZD_F_HUF_OK 8u      // a Huffman tree has been defined (ZdHufSave::tree is valid)
 #define ZD_F_LL_OK 16u
 #define ZD_F_ML_OK 32u
 #define ZD_F_OF_OK 64u
@@ -38,9 +37,23 @@ struct ZdWarp {
 #define ZD_F_ML_DEF 512u
 #define ZD_F_OF_DEF 1024u
 #define ZD_F_HAS_CK 2048u   // checksum field was read
-#define ZD_F_LIT_STAGED 4096u  // the frame's Huffman literals were decoded ahead (k_zd_huf_literals); where: ZD_HUF_STAGED
+#define ZD_F_LIT_STAGED 4096u  // the frame's Huffman literals were decoded ahead (k_zd_huf_literals); where: ZdHufSave::staged
 #define ZD_F_LIT_BAD 8192u     // ... and found corrupt
-#define ZD_HUF_STAGED 264u     // offset of that pointer in the lane's Huffman save area (a single-block frame saves no tree)
+
+// what a frame's Huffman literals leave for its later blocks; per lane of the fused kernel, in global scratch
+struct ZdHufSave {
+	const u8* tree;     // the description of the last tree the frame defined, for Treeless blocks (ZD_F_HUF_OK)
+	const u8* staged;   // the literals k_zd_huf_literals decoded ahead (ZD_F_LIT_STAGED)
+	u32 tree_n;         // the bytes the description may take
+};
+
+// the lane-private state of the FSE sequence decode (zd_lane_decode) of one block
+struct ZdSeqState {
+	ZsBack b;
+	u32 sl, so, sm;     // the LL, OF and ML states
+	u32 rep0, rep1, rep2;
+	u32 left;           // sequences left
+};
 
 // one frame's decoding state; lives in the registers of the frame's lane
 struct ZdLane {
@@ -49,14 +62,12 @@ struct ZdLane {
 	u64 n, ip, cap, opos, fcs;
 	u64 base;           // lowest output position a match may reach (0; the block's start for a split frame's block)
 	u32 status, flags, fcs_len, cksum;
-	u32 rep0, rep1, rep2;
 	u32 ll_log, ml_log, of_log;
 	// block in flight
 	const u8* blk;      // block body
 	u32 blk_n;
-	u32 nseq, nseq_left, seq_base;
-	ZsBack b;
-	u32 sl, so, sm;
+	u32 nseq, seq_base;
+	ZdSeqState seq;     // (the repeat offsets carry over from block to block)
 };
 
 template <typename T>
@@ -78,9 +89,9 @@ ZG_DEV ZdLane zd_bcast(const ZdLane& L, int f) {
 	U.flags = zd_bc(L.flags, f);
 	U.fcs_len = zd_bc(L.fcs_len, f);
 	U.cksum = zd_bc(L.cksum, f);
-	U.rep0 = zd_bc(L.rep0, f);
-	U.rep1 = zd_bc(L.rep1, f);
-	U.rep2 = zd_bc(L.rep2, f);
+	U.seq.rep0 = zd_bc(L.seq.rep0, f);
+	U.seq.rep1 = zd_bc(L.seq.rep1, f);
+	U.seq.rep2 = zd_bc(L.seq.rep2, f);
 	U.ll_log = zd_bc(L.ll_log, f);
 	U.ml_log = zd_bc(L.ml_log, f);
 	U.of_log = zd_bc(L.of_log, f);
@@ -88,16 +99,16 @@ ZG_DEV ZdLane zd_bcast(const ZdLane& L, int f) {
 	U.blk = zd_bc(L.blk, f);
 	U.blk_n = zd_bc(L.blk_n, f);
 	U.nseq = zd_bc(L.nseq, f);
-	U.nseq_left = zd_bc(L.nseq_left, f);
+	U.seq.left = zd_bc(L.seq.left, f);
 	U.seq_base = zd_bc(L.seq_base, f);
-	U.b.start = zd_bc(L.b.start, f);
-	U.b.ptr = zd_bc(L.b.ptr, f);
-	U.b.lo = zd_bc(L.b.lo, f);
-	U.b.hi = zd_bc(L.b.hi, f);
-	U.b.consumed = zd_bc(L.b.consumed, f);
-	U.sl = zd_bc(L.sl, f);
-	U.so = zd_bc(L.so, f);
-	U.sm = zd_bc(L.sm, f);
+	U.seq.b.start = zd_bc(L.seq.b.start, f);
+	U.seq.b.ptr = zd_bc(L.seq.b.ptr, f);
+	U.seq.b.lo = zd_bc(L.seq.b.lo, f);
+	U.seq.b.hi = zd_bc(L.seq.b.hi, f);
+	U.seq.b.consumed = zd_bc(L.seq.b.consumed, f);
+	U.seq.sl = zd_bc(L.seq.sl, f);
+	U.seq.so = zd_bc(L.seq.so, f);
+	U.seq.sm = zd_bc(L.seq.sm, f);
 	return U;
 }
 
@@ -172,8 +183,9 @@ ZG_DEV void zd_warp_match(u8* d, u32 off, u32 ml) {
 }
 
 // ---------------------------------------------------------------------------------------------
-// Huffman tree descriptions (RFC 8878 §4.2.1), read warp-wide (zd_read_huf_weights, zd_build_huf) or one per lane
-// (zd_read_huf_weights_lane, k_zd_huf_literals), both through the single-thread helpers below.
+// Huffman tree descriptions (RFC 8878 §4.2.1), each read on one lane (zd_read_huf_weights_lane, zd_huf_weights_check):
+// by lane 0 of the warp that decodes the block (zd_warp_huf_literals), or one per lane in k_zd_huf_literals.  The
+// table is then filled warp-wide (zd_huf_fill_table).
 
 // The description's size from its header byte: direct weights (*nw of them, as nibbles) or FSE-coded (*nw = 0).
 // Returns the bytes it takes (0 when they do not fit in n, or an FSE description is shorter than 2 bytes).
@@ -227,59 +239,8 @@ ZG_DEV u32 zd_huf_tree_check(u32 sum, u32 ones, u32& last) {
 	if (ones < 2 || (ones & 1)) return 0;  // as libzstd HUF_readStats
 	return maxbits;
 }
-// One step of a table fill: the symbol s of weight w (0: none) takes 2^(w-1) entries from `start`.  Short ranges are
-// written by the owning lane, long ones by the warp.  All lanes call.
-ZG_DEV void zd_huf_fill(u16* huf, u32 s, u32 w, u32 start, u32 maxbits) {
-	u32 lane = zg_lane();
-	u32 len = w ? 1u << (w - 1) : 0;
-	u32 entry = s | ((maxbits + 1 - w) << 8);
-	if (len > 0 && len < 32)
-		for (u32 k = 0; k < len; k++) huf[start + k] = (u16)entry;
-	u32 big = __ballot_sync(ZG_FULL, len >= 32);
-	while (big) {
-		int l = __ffs((int)big) - 1;
-		big &= big - 1;
-		u32 bs = __shfl_sync(ZG_FULL, start, l), bl = __shfl_sync(ZG_FULL, len, l), be = __shfl_sync(ZG_FULL, entry, l);
-		for (u32 k = lane; k < bl; k += 32) huf[bs + k] = (u16)be;
-	}
-}
-
-// Huffman tree description -> W->weights[0..nw) (the last weight is implied).  Returns bytes
-// consumed (0 on error).  All lanes call.
-ZG_DEV_NOINLINE u32 zd_read_huf_weights(ZdWarp* W, const u8* src, u32 n, u32* nw_out) {
-	u32 lane = zg_lane();
-	u32 nw;
-	u32 used = zd_huf_desc_size(src, n, &nw);
-	if (used == 0) return 0;
-	if (nw) {
-		for (u32 i = lane; i < nw; i += 32) zd_huf_direct_weights(src, i, W->weights);
-		__syncwarp();
-	} else {
-		u32 csz = used - 1;
-		if (lane == 0) {
-			u32 nsym = 0, log = 0;
-			u32 nc = zs_read_ncount(src + 1, csz, 6, 255, W->norm, &nsym, &log);
-			W->misc[0] = nc;
-			W->misc[1] = nsym;
-			W->misc[2] = log;
-		}
-		__syncwarp();
-		u32 nc = W->misc[0], nsym = W->misc[1], log = W->misc[2];
-		__syncwarp();
-		if (nc == 0 || nc >= csz) return 0;
-		zs_fse_build_dtable(W->tab, W->norm, nsym, log, W->next);
-		if (lane == 0) W->misc[0] = zd_huf_fse_weights(W->tab, log, src + 1 + nc, csz - nc, W->weights);
-		__syncwarp();
-		nw = W->misc[0];
-		__syncwarp();
-		if (nw == 0) return 0;
-	}
-	*nw_out = nw;
-	return used;
-}
-
-// The same on one lane: the description -> weights[0..nw).  `fse` (64 cells) and `list` (64 words, which may be
-// `weights` itself) are the lane's scratch for FSE-coded weights.
+// A tree description -> weights[0..nw) (the last weight is implied).  Returns the bytes it takes (0 on error).  `fse`
+// (64 cells) and `list` (64 words, which may be `weights` itself) are the lane's scratch for FSE-coded weights.
 ZG_DEV u32 zd_read_huf_weights_lane(const u8* src, u32 n, u8* weights, u32* fse, u32* list, u32* nw_out) {
 	u32 nw;
 	u32 used = zd_huf_desc_size(src, n, &nw);
@@ -331,58 +292,31 @@ ZG_DEV u32 zd_huf_weights_check(u8* weights, u32 nw, u16* start) {
 	return maxbits;
 }
 
-// W->weights[0..nw) -> huf (shared, 1 << maxbits entries).  Returns maxbits (0 on error).  All lanes call.
-ZG_DEV_NOINLINE u32 zd_build_huf(ZdWarp* W, u16* huf, u32 nw) {
+// weights[0..nsym) -> huf (1 << maxbits entries), all in shared memory: the symbols of weight w take 2^(w-1) entries
+// each, in symbol order from start[w] on (zd_huf_weights_check; start[w] is advanced).  A symbol's start is its weight's
+// plus the entries of the symbols of that weight before it (match_any over 32 symbols at a time).  Short ranges are
+// written by the owning lane, long ones by the warp.  All lanes call.
+ZG_DEV void zd_huf_fill_table(u16* huf, const u8* weights, u32 nsym, u16* start, u32 maxbits) {
 	u32 lane = zg_lane();
-	// weights -> last weight, ranks, per-symbol start index (serial, <= 256 symbols)
-	if (lane == 0) {
-		u32 sum = 0, maxbits = 0, last = 0;
-		bool ok = true;
-		u32 rank[13];
-		for (u32 i = 0; i < 13; i++) rank[i] = 0;
-		for (u32 i = 0; i < nw; i++) {
-			u32 w = W->weights[i];
-			if (w > 11) ok = false;
-			else {
-				if (w) sum += 1u << (w - 1);
-				rank[w]++;
-			}
+	for (u32 s0 = 0; s0 < nsym; s0 += 32) {
+		u32 s = s0 + lane, w = s < nsym ? weights[s] : 0;
+		u32 peers = __match_any_sync(ZG_FULL, w);
+		u32 len = w ? 1u << (w - 1) : 0;
+		u32 at = w ? start[w] + (u32)__popc(peers & zg_lanemask_lt()) * len : 0;
+		__syncwarp();
+		if (w && (peers & zg_lanemask_lt()) == 0) start[w] += (u32)__popc(peers) * len;
+		u32 entry = s | ((maxbits + 1 - w) << 8);
+		if (len > 0 && len < 32)
+			for (u32 k = 0; k < len; k++) huf[at + k] = (u16)entry;
+		u32 big = __ballot_sync(ZG_FULL, len >= 32);
+		while (big) {
+			int l = __ffs((int)big) - 1;
+			big &= big - 1;
+			u32 bs = __shfl_sync(ZG_FULL, at, l), bl = __shfl_sync(ZG_FULL, len, l), be = __shfl_sync(ZG_FULL, entry, l);
+			for (u32 k = lane; k < bl; k += 32) huf[bs + k] = (u16)be;
 		}
-		if (ok) maxbits = zd_huf_tree_check(sum, rank[1], last);
-		ok = maxbits != 0;
-		if (ok) {
-			W->weights[nw] = (u8)last;
-			rank[last]++;
-			u32 start = 0;
-			u32 rs[13];
-			for (u32 w = 1; w <= 11; w++) {
-				rs[w] = start;
-				start += rank[w] << (w - 1);
-			}
-			for (u32 i = 0; i <= nw; i++) {
-				u32 w = W->weights[i];
-				if (w) {
-					W->next[i] = (u16)rs[w];
-					rs[w] += 1u << (w - 1);
-				}
-			}
-		}
-		W->misc[0] = ok ? 1 : 0;
-		W->misc[1] = maxbits;
+		__syncwarp();
 	}
-	__syncwarp();
-	bool ok = W->misc[0] != 0;
-	u32 maxbits = W->misc[1];
-	__syncwarp();
-	if (!ok) return 0;
-	nw += 1;
-	for (u32 s0 = 0; s0 < nw; s0 += 32) {
-		u32 s = s0 + lane;
-		u32 w = s < nw ? W->weights[s] : 0;
-		zd_huf_fill(huf, s, w, w ? W->next[s] : 0, maxbits);
-	}
-	__syncwarp();
-	return maxbits;
 }
 
 // one Huffman stream, single thread.  Four symbols per refill of the bit container, stored as one aligned word (byte
@@ -488,16 +422,26 @@ ZG_DEV_NOINLINE bool zd_seq_table(ZdWarp* W, u32* slot, u32& log, u32& flags, u3
 	return (flags & ok_flag) != 0;  // Repeat_Mode: the slot (or the predefined flag) still holds the table
 }
 
+// The sequences bitstream p..end of a block and the three initial states.  Returns false when malformed.
+ZG_DEV bool zd_seq_start(ZdSeqState& s, const u8* p, const u8* end, u32 ll_log, u32 of_log, u32 ml_log) {
+	if (!zs_back_init(s.b, p, (u32)(end - p))) return false;
+	zs_back_reload(s.b);
+	s.sl = zs_back_read(s.b, ll_log);
+	s.so = zs_back_read(s.b, of_log);
+	s.sm = zs_back_read(s.b, ml_log);
+	return !zs_back_overflow(s.b);
+}
+
 // ---------------------------------------------------------------------------------------------
 ZG_DEV void zd_fail(ZdLane& U, u32 code) {
 	U.status = code;
 	U.flags &= ~ZD_F_ACTIVE;
-	U.nseq = U.nseq_left = 0;
+	U.nseq = U.seq.left = 0;
 }
 // end of frame: optional checksum field, content-size check
 ZG_DEV void zd_frame_finish(ZdLane& U) {
 	U.flags &= ~ZD_F_ACTIVE;
-	U.nseq = U.nseq_left = 0;
+	U.nseq = U.seq.left = 0;
 	if (U.flags & ZD_F_CKSUM) {
 		if (U.ip + 4 > U.n) {
 			U.status = ZS_E_SRC_SIZE;
@@ -510,44 +454,51 @@ ZG_DEV void zd_frame_finish(ZdLane& U) {
 	if (U.fcs_len && U.fcs != U.opos) U.status = ZS_E_CORRUPT;
 }
 
-// frame header (lane-private)
-ZG_DEV void zd_frame_header(ZdLane& L) {
-	const u8* src = L.src;
-	u64 n = L.n;
-	if (n < 6) return zd_fail(L, ZS_E_SRC_SIZE);
-	if (zg_ld32(src) != ZS_MAGIC) return zd_fail(L, ZS_E_PREFIX);
+// Frame_Header (RFC 8878 §3.1.1.1) of the frame src[0..n): where its first block starts, the content size (fcs_len
+// bytes of it were given, 0: none) and whether a Content_Checksum ends the frame (all 0 when the header is bad).
+// Returns a ZS_E_* code.  Single thread.
+struct ZdFrameHdr {
+	u64 ip, fcs;
+	u32 fcs_len, cksum;
+};
+ZG_DEV u32 zd_frame_header(const u8* src, u64 n, ZdFrameHdr& F) {
+	F.ip = F.fcs = 0;
+	F.fcs_len = F.cksum = 0;
+	if (n < 6) return ZS_E_SRC_SIZE;
+	if (zg_ld32(src) != ZS_MAGIC) return ZS_E_PREFIX;
 	u32 desc = src[4];
 	u32 fcs_flag = desc >> 6, single = (desc >> 5) & 1, checksum = (desc >> 2) & 1, did_flag = desc & 3;
-	if (desc & 8) return zd_fail(L, ZS_E_UNSUPPORTED);
+	if (desc & 8) return ZS_E_UNSUPPORTED;
 	u64 ip = 5;
 	u64 window = 0;
 	if (!single) {
 		u32 wd = src[ip++];
 		u32 wl = 10 + (wd >> 3);
-		if (wl > 31) return zd_fail(L, ZS_E_WINDOW);
+		if (wl > 31) return ZS_E_WINDOW;
 		window = ((u64)1 << wl) + ((((u64)1 << wl) >> 3) * (wd & 7));
 	}
 	if (did_flag) {
 		u32 dl = did_flag == 3 ? 4 : did_flag;
-		if (ip + dl > n) return zd_fail(L, ZS_E_SRC_SIZE);
+		if (ip + dl > n) return ZS_E_SRC_SIZE;
 		u32 did = 0;
 		for (u32 i = 0; i < dl; i++) did |= (u32)src[ip + i] << (8 * i);
 		ip += dl;
-		if (did) return zd_fail(L, ZS_E_DICT);
+		if (did) return ZS_E_DICT;
 	}
 	u32 fcs_len = fcs_flag == 0 ? single : fcs_flag == 1 ? 2 : fcs_flag == 2 ? 4 : 8;
-	if (ip + fcs_len > n) return zd_fail(L, ZS_E_SRC_SIZE);
+	if (ip + fcs_len > n) return ZS_E_SRC_SIZE;
 	u64 fcs = 0;
 	for (u32 i = 0; i < fcs_len; i++) fcs |= (u64)src[ip + i] << (8 * i);
 	if (fcs_len == 2) fcs += 256;
 	ip += fcs_len;
 	// libzstd's streaming decoder (what zstd_iterator.rs:29 creates) refuses windows > 2^27
 	// ("Frame requires too much memory for decoding", SURVEY.md App. C)
-	if ((single ? fcs : window) > ((u64)1 << 27)) return zd_fail(L, ZS_E_WINDOW);
-	L.ip = ip;
-	L.fcs = fcs;
-	L.fcs_len = fcs_len;
-	if (checksum) L.flags |= ZD_F_CKSUM;
+	if ((single ? fcs : window) > ((u64)1 << 27)) return ZS_E_WINDOW;
+	F.ip = ip;
+	F.fcs = fcs;
+	F.fcs_len = fcs_len;
+	F.cksum = checksum;
+	return ZS_OK;
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -610,29 +561,86 @@ ZG_DEV bool zd_lit_header(const u8* src, u32 n, ZdLitHdr& h) {
 #define ZD_LIT_BAD (~0ull - 1ull)  // ... decoded ahead and corrupt
 ZG_DEV bool zd_single_huf_section(const u8* archive, u64 archive_len, u64 fo, u64 fl, u64& at, u32& regen) {
 	if (fo > archive_len || fl > archive_len - fo) return false;
-	ZdLane L;
-	L.src = archive + fo;
-	L.n = fl;
-	L.status = ZS_OK;
-	L.flags = 0;
-	L.ip = L.fcs = 0;
-	L.fcs_len = 0;
-	zd_frame_header(L);
-	if (L.status != ZS_OK || L.ip + 3 > fl) return false;
-	u32 bh = zg_ld24(L.src + L.ip), bsize = bh >> 3;
-	if ((bh & 7u) != 5u || bsize > ZS_BLOCK_MAX || L.ip + 3 + bsize > fl) return false;  // Last_Block, Compressed_Block
+	const u8* src = archive + fo;
+	ZdFrameHdr F;
+	if (zd_frame_header(src, fl, F) != ZS_OK || F.ip + 3 > fl) return false;
+	u32 bh = zg_ld24(src + F.ip), bsize = bh >> 3;
+	if ((bh & 7u) != 5u || bsize > ZS_BLOCK_MAX || F.ip + 3 + bsize > fl) return false;  // Last_Block, Compressed_Block
 	ZdLitHdr h;
-	if (!zd_lit_header(L.src + L.ip + 3, bsize, h) || h.ltype != 2) return false;
-	at = fo + L.ip + 3;
+	if (!zd_lit_header(src + F.ip + 3, bsize, h) || h.ltype != 2) return false;
+	at = fo + F.ip + 3;
 	regen = h.regen;
 	return true;
 }
 
+// Literals_Section_Header and Sequences_Section_Header of a compressed block (RFC 8878 §3.1.1.3): Number_of_Sequences
+// (at most `maxseq`) and Symbol_Compression_Modes.  Returns false when malformed.  Single thread.
+struct ZdSect {
+	ZdLitHdr h;
+	u32 nseq, modes;
+	const u8* tables;   // first table description (after the modes byte)
+};
+ZG_DEV bool zd_sections(const u8* src, u32 n, u32 maxseq, ZdSect& S) {
+	if (!zd_lit_header(src, n, S.h)) return false;
+	const u8* end = src + n;
+	const u8* p = src + S.h.hdr + S.h.comp;
+	if (p >= end) return false;
+	u32 c0 = p[0];
+	if (c0 < 128) {
+		S.nseq = c0;
+		p += 1;
+	} else if (c0 < 255) {
+		if (end - p < 2) return false;
+		S.nseq = ((c0 - 128) << 8) + p[1];
+		p += 2;
+	} else {
+		if (end - p < 3) return false;
+		S.nseq = (u32)p[1] + ((u32)p[2] << 8) + 0x7F00;
+		p += 3;
+	}
+	S.modes = 0;
+	if (S.nseq == 0) {
+		S.tables = p;
+		return p == end;
+	}
+	if (p >= end) return false;
+	S.modes = *p++;
+	S.tables = p;
+	return (S.modes & 3) == 0 && S.nseq <= maxseq;
+}
+
+// Huffman literals of one block (uniform in the warp) into dst: lp = the section after its header, `tree` / `tn` = the
+// tree description and the bytes it may take (for a Huffman_Literals_Block its own, at lp; for a Treeless one the
+// description of the block that last defined a tree).  Lane 0 reads the tree.  Returns a ZS_E_* code.
+ZG_DEV_NOINLINE u32 zd_warp_huf_literals(ZdWarp* W, const u8* tree, u32 tn, const u8* lp, const ZdLitHdr& h, u8* dst) {
+	u32 lane = zg_lane();
+	u32 used = 0, nw = 0, bits = 0;
+	if (lane == 0) {
+		used = zd_read_huf_weights_lane(tree, tn, W->weights, W->tab, (u32*)W->weights, &nw);
+		bits = used ? zd_huf_weights_check(W->weights, nw, W->next) : 0;
+	}
+	__syncwarp();
+	bits = __shfl_sync(ZG_FULL, bits, 0);
+	if (bits == 0) return ZS_E_CORRUPT;
+	used = __shfl_sync(ZG_FULL, used, 0);
+	nw = __shfl_sync(ZG_FULL, nw, 0);
+	zd_huf_fill_table(W->huf, W->weights, nw + 1, W->next, bits);
+	const u8* lend = lp + h.comp;
+	if (h.ltype == 2) lp += used;
+	const u8* sp;
+	u32 sn, first, cnt;
+	if (!zd_huf_split(lp, lend, h.regen, h.streams, lane, sp, sn, first, cnt)) return ZS_E_CORRUPT;
+	bool ok = true;
+	if (lane < h.streams) ok = zd_huf_stream(W->huf, bits, sp, sn, dst + first, cnt);
+	if (!__all_sync(ZG_FULL, ok)) return ZS_E_CORRUPT;
+	__syncwarp();
+	return ZS_OK;
+}
+
 // The block's literals (uniform in the warp): Raw -> pointer into the block, RLE -> the byte,
 // Huffman -> decoded into litbuf.  Returns a ZS_E_* code.
-ZG_DEV_NOINLINE u32 zd_literals(ZdWarp* W, u32& flags, const u8* src, const ZdLitHdr& h, bool last, u8* litbuf, u8* hufsave, const u8*& lit,
+ZG_DEV_NOINLINE u32 zd_literals(ZdWarp* W, u32& flags, const u8* src, const ZdLitHdr& h, u8* litbuf, ZdHufSave* save, const u8*& lit,
                        bool& lit_rle, u32& rle_byte) {
-	u32 lane = zg_lane();
 	lit_rle = false;
 	rle_byte = 0;
 	if (h.ltype == 0) {
@@ -648,44 +656,25 @@ ZG_DEV_NOINLINE u32 zd_literals(ZdWarp* W, u32& flags, const u8* src, const ZdLi
 	if (flags & (ZD_F_LIT_STAGED | ZD_F_LIT_BAD)) {  // a single-block frame's literals, decoded ahead by k_zd_huf_literals
 		if (flags & ZD_F_LIT_BAD) return ZS_E_CORRUPT;
 		flags |= ZD_F_HUF_OK;
-		lit = *(const u8* const*)(hufsave + ZD_HUF_STAGED);
+		lit = save->staged;
 		return ZS_OK;
 	}
 	const u8* lp = src + h.hdr;
-	const u8* lend = lp + h.comp;
-	u32 regen = h.regen;
-	u32 huf_bits;
-	if (h.ltype == 2) {
-		u32 nw = 0;
-		u32 used = zd_read_huf_weights(W, lp, h.comp, &nw);
-		if (used == 0) return ZS_E_CORRUPT;
-		if (!last) {  // a later Treeless block may need this tree again
-			for (u32 i = lane; i < nw; i += 32) hufsave[i] = W->weights[i];
-			if (lane == 0) {
-				hufsave[256] = (u8)nw;
-				hufsave[257] = (u8)(nw >> 8);
-			}
+	const u8* tree = lp;
+	u32 tn = h.comp;
+	if (h.ltype == 2) {  // a later Treeless block reads this description again
+		if (zg_lane() == 0) {
+			save->tree = lp;
+			save->tree_n = h.comp;
 		}
-		huf_bits = zd_build_huf(W, W->huf, nw);
-		if (huf_bits == 0) return ZS_E_CORRUPT;
-		flags |= ZD_F_HUF_OK;
-		lp += used;
 	} else {
 		if (!(flags & ZD_F_HUF_OK)) return ZS_E_CORRUPT;
-		u32 nw = (u32)hufsave[256] | ((u32)hufsave[257] << 8);
-		__syncwarp();
-		for (u32 i = lane; i < nw; i += 32) W->weights[i] = hufsave[i];
-		__syncwarp();
-		huf_bits = zd_build_huf(W, W->huf, nw);
-		if (huf_bits == 0) return ZS_E_CORRUPT;
+		tree = save->tree;
+		tn = save->tree_n;
 	}
-	const u8* sp;
-	u32 sn, first, cnt;
-	if (!zd_huf_split(lp, lend, regen, h.streams, lane, sp, sn, first, cnt)) return ZS_E_CORRUPT;
-	bool ok = true;
-	if (lane < h.streams) ok = zd_huf_stream(W->huf, huf_bits, sp, sn, litbuf + first, cnt);
-	if (!__all_sync(ZG_FULL, ok)) return ZS_E_CORRUPT;
-	__syncwarp();
+	u32 r = zd_warp_huf_literals(W, tree, tn, lp, h, litbuf);
+	if (r) return r;
+	flags |= ZD_F_HUF_OK;
 	lit = litbuf;
 	return ZS_OK;
 }
@@ -696,35 +685,16 @@ ZG_DEV_NOINLINE u32 zd_literals(ZdWarp* W, u32& flags, const u8* src, const ZdLi
 // ZD_DEFER = the sequence arena is full (nothing consumed), else a ZS_E_* code + 1.
 #define ZD_DEFER 1u
 #define ZD_ERR(c) ((c) + 1u)
-ZG_DEV u32 zd_block_setup(ZdWarp* W, ZdLane& U, const u8* src, u32 n, bool last, u32* slot, u32& arena_used, u8* litbuf, u8* hufsave) {
-	ZdLitHdr h;
-	if (!zd_lit_header(src, n, h)) return ZD_ERR(ZS_E_CORRUPT);
-	const u8* end = src + n;
-	const u8* p = src + h.hdr + h.comp;
-	// ---- sequences section header ----
-	if (p >= end) return ZD_ERR(ZS_E_CORRUPT);
-	u32 nseq;
-	{
-		u32 c0 = p[0];
-		if (c0 < 128) {
-			nseq = c0;
-			p += 1;
-		} else if (c0 < 255) {
-			if (end - p < 2) return ZD_ERR(ZS_E_CORRUPT);
-			nseq = ((c0 - 128) << 8) + p[1];
-			p += 2;
-		} else {
-			if (end - p < 3) return ZD_ERR(ZS_E_CORRUPT);
-			nseq = (u32)p[1] + ((u32)p[2] << 8) + 0x7F00;
-			p += 3;
-		}
-	}
-	if (nseq == 0) {
-		if (p != end) return ZD_ERR(ZS_E_CORRUPT);
+ZG_DEV u32 zd_block_setup(ZdWarp* W, ZdLane& U, const u8* src, u32 n, u32* slot, u32& arena_used, u8* litbuf, ZdHufSave* save) {
+	ZdSect S;
+	// (the arena bounds the count: > 131072 sequences cannot come from a 128 KiB block)
+	if (!zd_sections(src, n, ZD_SEQ_ARENA, S)) return ZD_ERR(ZS_E_CORRUPT);
+	const ZdLitHdr& h = S.h;
+	if (S.nseq == 0) {
 		const u8* lit;
 		bool lit_rle;
 		u32 rle_byte;
-		u32 r = zd_literals(W, U.flags, src, h, last, litbuf, hufsave, lit, lit_rle, rle_byte);
+		u32 r = zd_literals(W, U.flags, src, h, litbuf, save, lit, lit_rle, rle_byte);
 		if (r) return ZD_ERR(r);
 		if (U.opos + h.regen > U.cap) return ZD_ERR(ZS_E_DST_SMALL);
 		if (h.regen) {
@@ -732,37 +702,31 @@ ZG_DEV u32 zd_block_setup(ZdWarp* W, ZdLane& U, const u8* src, u32 n, bool last,
 			else zg_warp_copy(U.out + U.opos, lit, h.regen);
 		}
 		U.opos += h.regen;
-		U.nseq = U.nseq_left = 0;
+		U.nseq = U.seq.left = 0;
 		__syncwarp();
 		return 0;
 	}
-	if (nseq > ZD_SEQ_ARENA) return ZD_ERR(ZS_E_CORRUPT);  // > 131072 sequences cannot come from a 128 KiB block
-	if (arena_used + nseq > ZD_SEQ_ARENA) return ZD_DEFER;    // (an empty arena always fits a block)
-	if (p >= end) return ZD_ERR(ZS_E_CORRUPT);
-	u32 modes = *p++;
-	if (modes & 3) return ZD_ERR(ZS_E_CORRUPT);
+	if (arena_used + S.nseq > ZD_SEQ_ARENA) return ZD_DEFER;  // (an empty arena always fits a block)
+	const u8* end = src + n;
+	const u8* p = S.tables;
+	u32 modes = S.modes;
 	if (!zd_seq_table(W, slot, U.ll_log, U.flags, ZD_F_LL_OK, ZD_F_LL_DEF, (modes >> 6) & 3, p, end, ZS_LL_MAXLOG, 35, 6)) return ZD_ERR(ZS_E_CORRUPT);
 	if (!zd_seq_table(W, slot + 1024, U.of_log, U.flags, ZD_F_OF_OK, ZD_F_OF_DEF, (modes >> 4) & 3, p, end, ZS_OF_MAXLOG, 31, 5)) return ZD_ERR(ZS_E_CORRUPT);
 	if (!zd_seq_table(W, slot + 512, U.ml_log, U.flags, ZD_F_ML_OK, ZD_F_ML_DEF, (modes >> 2) & 3, p, end, ZS_ML_MAXLOG, 52, 6)) return ZD_ERR(ZS_E_CORRUPT);
-	// bitstream + the three initial states (uniform here; the frame's lane keeps them)
-	if (!zs_back_init(U.b, p, (u32)(end - p))) return ZD_ERR(ZS_E_CORRUPT);
-	zs_back_reload(U.b);
-	U.sl = zs_back_read(U.b, U.ll_log);
-	U.so = zs_back_read(U.b, U.of_log);
-	U.sm = zs_back_read(U.b, U.ml_log);
-	if (zs_back_overflow(U.b)) return ZD_ERR(ZS_E_CORRUPT);
-	U.nseq = U.nseq_left = nseq;
+	// (uniform here; the frame's lane keeps the state)
+	if (!zd_seq_start(U.seq, p, end, U.ll_log, U.of_log, U.ml_log)) return ZD_ERR(ZS_E_CORRUPT);
+	U.nseq = U.seq.left = S.nseq;
 	U.seq_base = arena_used;
 	U.blk = src;
 	U.blk_n = n;
-	arena_used += nseq;
+	arena_used += S.nseq;
 	__syncwarp();
 	return 0;
 }
 
 // Advance the frame viewed by U (uniform) through its blocks until one with sequences is ready for
 // phase B, the frame ends, fails, or has to wait for arena space.
-ZG_DEV void zd_setup_frame(ZdWarp* W, ZdLane& U, u32* slot, u32& arena_used, u8* litbuf, u8* hufsave) {
+ZG_DEV void zd_setup_frame(ZdWarp* W, ZdLane& U, u32* slot, u32& arena_used, u8* litbuf, ZdHufSave* save) {
 	for (;;) {
 		if (U.ip + 3 > U.n) return zd_fail(U, ZS_E_SRC_SIZE);
 		u32 bh = zg_ld24(U.src + U.ip);
@@ -786,7 +750,7 @@ ZG_DEV void zd_setup_frame(ZdWarp* W, ZdLane& U, u32* slot, u32& arena_used, u8*
 		} else {
 			if (bsize > ZS_BLOCK_MAX) return zd_fail(U, ZS_E_CORRUPT);
 			if (body + bsize > U.n) return zd_fail(U, ZS_E_SRC_SIZE);
-			u32 r = zd_block_setup(W, U, U.src + body, bsize, last != 0, slot, arena_used, litbuf, hufsave);
+			u32 r = zd_block_setup(W, U, U.src + body, bsize, slot, arena_used, litbuf, save);
 			if (r == ZD_DEFER) return;
 			if (r) return zd_fail(U, r - 1u);
 			U.ip = body + bsize;
@@ -801,13 +765,25 @@ ZG_DEV void zd_setup_frame(ZdWarp* W, ZdLane& U, u32* slot, u32& arena_used, u8*
 }
 
 // ---------------------------------------------------------------------------------------------
-// Phase B, lane-private: decode up to `cnt` sequences of this lane's block and append them, packed,
-// to dst.  The caller keeps all lanes in step (cnt is bounded) so that the warp stays converged.
-ZG_DEV bool zd_lane_decode(ZdLane& L, u32 cnt, const u32* llt, const u32* mlt, const u32* oft, u64* dst) {
-	ZsBack b = L.b;
-	u32 sl = L.sl, so = L.so, sm = L.sm;
-	u32 rep0 = L.rep0, rep1 = L.rep1, rep2 = L.rep2;
-	u32 left = L.nseq_left;
+// The fused kernel's policy for zd_lane_decode: offsets beyond 2^28 exceed every window this decoder accepts; an
+// offset of 0 only arises from a corrupt stream or from the unknown repeat-offset history of a split frame's block (then
+// the block is not independent); lengths are < 2^18 by construction.  No bookkeeping.
+struct ZdSeqPlain {
+	static ZG_DEV bool bad(u32 off, bool) { return off - 1u >= ZD_OFF_MAX; }
+	ZG_DEV void seq(u32, u32, u32) {}
+};
+
+// Phase B, lane-private: decode up to `cnt` sequences of this lane's block and append them, packed
+// (offset:28 | litLength:18 | matchLength:18), to dst.  The caller keeps all lanes in step (cnt is bounded) so that the
+// warp stays converged.  POL::bad(off, fresh) checks an offset (fresh: not a repeat code), P.seq(off, ll, ml) follows
+// every sequence.  S and P are written back only when the call succeeds.
+template <class POL>
+ZG_DEV bool zd_lane_decode(ZdSeqState& S, POL& P, u32 cnt, const u32* llt, const u32* mlt, const u32* oft, u64* dst) {
+	ZsBack b = S.b;
+	u32 sl = S.sl, so = S.so, sm = S.sm;
+	u32 rep0 = S.rep0, rep1 = S.rep1, rep2 = S.rep2;
+	u32 left = S.left;
+	POL pol = P;
 	ZsBelow ahead = {0, 0};
 	zs_below_fetch(b, ahead);
 	u32 bad = 0;  // checked once per call: a bad sequence only poisons values, never an address (states stay inside their tables)
@@ -849,10 +825,8 @@ ZG_DEV bool zd_lane_decode(ZdLane& L, u32 cnt, const u32* llt, const u32* mlt, c
 				rep0 = off;
 			}
 		}
-		// offsets beyond 2^28 exceed every window this decoder accepts; an offset of 0 only arises from a corrupt stream
-		// or from the unknown repeat-offset history of a split frame's block (then the block is not independent);
-		// lengths are < 2^18 by construction
-		bad |= (off - 1u >= ZD_OFF_MAX) ? 1u : 0u;
+		bad |= POL::bad(off, ofv > 3) ? 1u : 0u;
+		pol.seq(off, ll, ml);
 		dst[k] = (u64)off | ((u64)ll << 28) | ((u64)ml << 46);
 	}
 	if (bad || zs_back_overflow(b)) return false;
@@ -861,14 +835,15 @@ ZG_DEV bool zd_lane_decode(ZdLane& L, u32 cnt, const u32* llt, const u32* mlt, c
 		zs_back_reload(b);
 		if (!zs_back_finished(b)) return false;
 	}
-	L.b = b;
-	L.sl = sl;
-	L.so = so;
-	L.sm = sm;
-	L.rep0 = rep0;
-	L.rep1 = rep1;
-	L.rep2 = rep2;
-	L.nseq_left = left;
+	S.b = b;
+	S.sl = sl;
+	S.so = so;
+	S.sm = sm;
+	S.rep0 = rep0;
+	S.rep1 = rep1;
+	S.rep2 = rep2;
+	S.left = left;
+	P = pol;
 	return true;
 }
 
@@ -1019,13 +994,13 @@ ZG_DEV u32 zd_exec_row(u64 sq_lane, u32 cnt, const POL& P, u64& o_io, u64 base, 
 }
 
 // Phase C for the block in flight of the frame viewed by U (uniform): literals, then all sequences.
-ZG_DEV void zd_exec_block(ZdWarp* W, ZdLane& U, const u64* seqs, u8* litbuf, u8* hufsave) {
+ZG_DEV void zd_exec_block(ZdWarp* W, ZdLane& U, const u64* seqs, u8* litbuf, ZdHufSave* save) {
 	ZdLitHdr h;
 	zd_lit_header(U.blk, U.blk_n, h);  // validated in phase A
 	const u8* lit;
 	bool lit_rle;
 	u32 rle_byte;
-	u32 r = zd_literals(W, U.flags, U.blk, h, (U.flags & ZD_F_LAST) != 0, litbuf, hufsave, lit, lit_rle, rle_byte);
+	u32 r = zd_literals(W, U.flags, U.blk, h, litbuf, save, lit, lit_rle, rle_byte);
 	if (r) return zd_fail(U, r);
 	u64 o = U.opos;
 	u32 lpos = 0;

@@ -85,19 +85,13 @@ ZG_DEV u32 zds_resolve(u32 v, u32 r0, u32 r1, u32 r2) {
 ZG_DEV u64 zds_walk(const u8* archive, u64 archive_len, u64 fo, u64 fl, u64 ul, u64 oo, u64 out_cap, u64 split_min, u32 k, ZdsBlk* blk,
                     u64* tail) {
 	if (ul < split_min || fo > archive_len || fl > archive_len - fo || oo > out_cap || ul > out_cap - oo) return 0;
-	ZdLane L;
-	L.src = archive + fo;
-	L.n = fl;
-	L.status = ZS_OK;
-	L.flags = 0;
-	L.ip = L.fcs = 0;
-	L.fcs_len = 0;
-	zd_frame_header(L);
-	if (L.status != ZS_OK || (L.fcs_len && L.fcs != ul)) return 0;
-	u64 ip = L.ip, nb = 0;
+	const u8* src = archive + fo;
+	ZdFrameHdr F;
+	if (zd_frame_header(src, fl, F) != ZS_OK || (F.fcs_len && F.fcs != ul)) return 0;
+	u64 ip = F.ip, nb = 0;
 	for (;;) {
 		if (ip + 3 > fl) return 0;
-		u32 bh = zg_ld24(L.src + ip);
+		u32 bh = zg_ld24(src + ip);
 		u32 last = bh & 1, type = (bh >> 1) & 3, bsize = bh >> 3;
 		if (type == 3 || bsize > ZS_BLOCK_MAX) return 0;
 		u64 body = type == 1 ? 1 : bsize;
@@ -179,40 +173,7 @@ k_zds_emit(const u8* __restrict__ archive, u64 archive_len, const u64* __restric
 }
 
 // ---------------------------------------------------------------------------------------------
-// 2. section headers of one compressed block (single thread).  Returns false when malformed.
-struct ZdsSect {
-	ZdLitHdr h;
-	u32 nseq, modes;
-	const u8* tables;   // first table description (after the modes byte)
-};
-ZG_DEV bool zds_sections(const u8* src, u32 n, ZdsSect& S) {
-	if (!zd_lit_header(src, n, S.h)) return false;
-	const u8* end = src + n;
-	const u8* p = src + S.h.hdr + S.h.comp;
-	if (p >= end) return false;
-	u32 c0 = p[0];
-	if (c0 < 128) {
-		S.nseq = c0;
-		p += 1;
-	} else if (c0 < 255) {
-		if (end - p < 2) return false;
-		S.nseq = ((c0 - 128) << 8) + p[1];
-		p += 2;
-	} else {
-		if (end - p < 3) return false;
-		S.nseq = (u32)p[1] + ((u32)p[2] << 8) + 0x7F00;
-		p += 3;
-	}
-	S.modes = 0;
-	if (S.nseq == 0) {
-		S.tables = p;
-		return p == end;
-	}
-	if (p >= end) return false;
-	S.modes = *p++;
-	S.tables = p;
-	return (S.modes & 3) == 0 && S.nseq <= ZDS_MAXSEQ;
-}
+// 2. section headers of one compressed block (thread per block)
 __global__ void __launch_bounds__(128)
 k_zds_modes(const u8* __restrict__ archive, const u64* __restrict__ off, ZdsBlk* __restrict__ blk, u64 nblocks) {
 	u64 g = (u64)blockIdx.x * blockDim.x + threadIdx.x;
@@ -221,8 +182,8 @@ k_zds_modes(const u8* __restrict__ archive, const u64* __restrict__ off, ZdsBlk*
 	u32 type = (B.hdr >> 1) & 3, bsize = B.hdr >> 3;
 	u32 info = 0, nseq = 0, regen = 0;
 	if (type == 2) {
-		ZdsSect S;
-		if (bsize == 0 || !zds_sections(archive + off[B.k] + B.ip + 3, bsize, S)) info = ZDS_I_BAD;
+		ZdSect S;
+		if (bsize == 0 || !zd_sections(archive + off[B.k] + B.ip + 3, bsize, ZDS_MAXSEQ, S)) info = ZDS_I_BAD;
 		else {
 			info = S.h.ltype | (S.nseq ? ZDS_I_SEQ : 0u) | (S.modes << 8);
 			nseq = S.nseq;
@@ -298,8 +259,8 @@ ZG_DEV bool zds_table(ZdWarp* W, u32* slot, u32& log, u32& flags, u32 ok_flag, u
                       const u8* fsrc, u32 fn, u32 maxlog, u32 maxsym, u32 def_log) {
 	if (mode != 3) return zd_seq_table(W, slot, log, flags, ok_flag, def_flag, mode, p, end, maxlog, maxsym, def_log);
 	if (!fsrc) return false;  // Repeat_Mode with nothing to repeat
-	ZdsSect F;
-	if (!zds_sections(fsrc, fn, F) || F.nseq == 0) return false;
+	ZdSect F;
+	if (!zd_sections(fsrc, fn, ZDS_MAXSEQ, F) || F.nseq == 0) return false;
 	const u8* q = F.tables;
 	const u8* qend = fsrc + fn;
 	// skip the descriptions in front of table t (order LL, OF, ML)
@@ -325,98 +286,16 @@ ZG_DEV bool zds_table(ZdWarp* W, u32* slot, u32& log, u32& flags, u32 ok_flag, u
 	return zd_seq_table(W, slot, log, flags, ok_flag, def_flag, fm, q, qend, maxlog, maxsym, def_log);
 }
 
-// Huffman literals of one block into dst (uniform).  `tsrc`/`tn`: the block whose tree a Treeless block uses.
-ZG_DEV_NOINLINE u32 zds_literals(ZdWarp* W, const u8* src, const ZdLitHdr& h, const u8* tsrc, u32 tn, u8* dst) {
-	u32 lane = zg_lane();
-	const u8* lp = src + h.hdr;
-	const u8* lend = lp + h.comp;
-	u32 nw = 0, huf_bits;
-	if (h.ltype == 2) {
-		u32 used = zd_read_huf_weights(W, lp, h.comp, &nw);
-		if (used == 0) return ZS_E_CORRUPT;
-		lp += used;
-	} else {
-		ZdLitHdr th;
-		if (!tsrc || !zd_lit_header(tsrc, tn, th) || th.ltype != 2) return ZS_E_CORRUPT;
-		if (zd_read_huf_weights(W, tsrc + th.hdr, th.comp, &nw) == 0) return ZS_E_CORRUPT;
-	}
-	huf_bits = zd_build_huf(W, W->huf, nw);
-	if (huf_bits == 0) return ZS_E_CORRUPT;
-	const u8* sp;
-	u32 sn, first, cnt;
-	if (!zd_huf_split(lp, lend, h.regen, h.streams, lane, sp, sn, first, cnt)) return ZS_E_CORRUPT;
-	bool ok = true;
-	if (lane < h.streams) ok = zd_huf_stream(W->huf, huf_bits, sp, sn, dst + first, cnt);
-	if (!__all_sync(ZG_FULL, ok)) return ZS_E_CORRUPT;
-	__syncwarp();
-	return ZS_OK;
-}
-
-// the lane-private state of one block in the entropy stage
-struct ZdsLane {
-	ZsBack b;
-	u32 sl, so, sm;
-	u32 ll_log, ml_log, of_log;
-	u32 flags;          // ZD_F_*_DEF
-	u32 nseq, left;
-	u32 status;
-	u32 rep0, rep1, rep2;
+// zd_lane_decode's policy in the entropy stage: offsets checked against the window, and how far the block reaches
+struct ZdsBook {
 	u32 pos, lit_used;  // bytes regenerated / literals consumed by the sequences so far
 	i32 reach;          // furthest a concrete offset went below the block's first byte
 	u32 sym;            // a symbolic offset was used
-};
-
-// `cnt` sequences of this lane's block -> dst, packed like the fused decoder's (offset:28 | litLength:18 | matchLength:18);
-// the loop body is zd_lane_decode's, with the offsets checked against the window and the block's reach tracked
-ZG_DEV bool zds_lane_decode(ZdsLane& L, u32 cnt, const u32* llt, const u32* mlt, const u32* oft, u64* dst) {
-	ZsBack b = L.b;
-	u32 sl = L.sl, so = L.so, sm = L.sm;
-	u32 rep0 = L.rep0, rep1 = L.rep1, rep2 = L.rep2;
-	u32 left = L.left, pos = L.pos, lit_used = L.lit_used, sym = L.sym;
-	i32 reach = L.reach;
-	ZsBelow ahead = {0, 0};
-	zs_below_fetch(b, ahead);
-	u32 bad = 0;
-	for (u32 k = 0; k < cnt; k++) {
-		u32 oe = oft[so], me = mlt[sm], le = llt[sl];
-		zs_back_reload_ahead(b, ahead);
-		u32 oc = oe & 0xff;
-		u32 mp = ZS_ML_PACK[me & 0xff], lp = ZS_LL_PACK[le & 0xff];
-		u32 ofv = (1u << oc) + zs_back_read(b, oc);
-		u32 used = oc;
-		if (oc > 24) {
-			zs_back_reload_ahead(b, ahead);
-			used = 0;
-		}
-		u32 mb = mp >> 24, lb = lp >> 24;
-		u32 ml = (mp & 0xffffffu) + zs_back_read(b, mb);
-		u32 ll = (lp & 0xffffffu) + zs_back_read(b, lb);
-		used += mb + lb;
-		if (left - k > 1) {
-			if (used > 30) zs_back_reload_ahead(b, ahead);
-			sl = (le >> 16) + zs_back_read(b, (le >> 8) & 0xff);
-			sm = (me >> 16) + zs_back_read(b, (me >> 8) & 0xff);
-			so = (oe >> 16) + zs_back_read(b, (oe >> 8) & 0xff);
-		}
-		u32 off;
-		if (ofv > 3) {
-			off = ofv - 3;
-			bad |= off > ZDS_WIN_MAX ? 1u : 0u;  // beyond every window this decoder accepts (and the symbolic range starts here)
-			rep2 = rep1;
-			rep1 = rep0;
-			rep0 = off;
-		} else {
-			u32 idx = ofv - 1 + (ll == 0 ? 1 : 0);
-			off = idx == 0 ? rep0 : idx == 1 ? rep1 : idx == 2 ? rep2 : rep0 - 1u;
-			if (idx > 1) rep2 = rep1;
-			if (idx > 0) {
-				rep1 = rep0;
-				rep0 = off;
-			}
-			// "rep0 - 1" of a concrete 1 is no offset; of a symbolic value it stays symbolic as long as the block has
-			// fewer than 2^25 sequences (it has at most ZDS_MAXSEQ)
-			bad |= off == 0u ? 1u : 0u;
-		}
+	// a new offset beyond every window this decoder accepts (the symbolic range starts there); a repeat of 0: "rep0 - 1"
+	// of a concrete 1 is no offset, of a symbolic value it stays symbolic as long as the block has fewer than 2^25
+	// sequences (it has at most ZDS_MAXSEQ)
+	static ZG_DEV bool bad(u32 off, bool fresh) { return fresh ? off > ZDS_WIN_MAX : off == 0u; }
+	ZG_DEV void seq(u32 off, u32 ll, u32 ml) {
 		pos += ll;
 		lit_used += ll;
 		bool s = zds_is_sym(off);
@@ -424,28 +303,18 @@ ZG_DEV bool zds_lane_decode(ZdsLane& L, u32 cnt, const u32* llt, const u32* mlt,
 		i32 r = (i32)off - (i32)pos;
 		reach = (!s && r > reach) ? r : reach;
 		pos += ml;
-		dst[k] = (u64)off | ((u64)ll << 28) | ((u64)ml << 46);
 	}
-	if (bad || zs_back_overflow(b)) return false;
-	left -= cnt;
-	if (left == 0) {
-		zs_back_reload(b);
-		if (!zs_back_finished(b)) return false;
-	}
-	L.b = b;
-	L.sl = sl;
-	L.so = so;
-	L.sm = sm;
-	L.rep0 = rep0;
-	L.rep1 = rep1;
-	L.rep2 = rep2;
-	L.left = left;
-	L.pos = pos;
-	L.lit_used = lit_used;
-	L.reach = reach;
-	L.sym = sym;
-	return true;
-}
+};
+
+// the lane-private state of one block in the entropy stage
+struct ZdsLane {
+	ZdSeqState seq;     // (the repeat offsets start symbolic)
+	ZdsBook book;
+	u32 ll_log, ml_log, of_log;
+	u32 flags;          // ZD_F_*_DEF
+	u32 nseq;
+	u32 status;
+};
 
 struct ZdsJob {
 	const u8* archive;
@@ -494,19 +363,20 @@ k_zds_entropy(ZdsJob J, u32* tabs, u32* queue, u32 want) {
 		if (mine) B = J.blk[g];
 		u32 type = (B.hdr >> 1) & 3, bsize = B.hdr >> 3;
 		ZdsLane L;
-		L.b.start = L.b.ptr = J.archive;
-		L.b.lo = L.b.hi = L.b.consumed = 0;
-		L.sl = L.so = L.sm = 0;
+		L.seq.b.start = L.seq.b.ptr = J.archive;
+		L.seq.b.lo = L.seq.b.hi = L.seq.b.consumed = 0;
+		L.seq.sl = L.seq.so = L.seq.sm = 0;
+		L.seq.rep0 = zds_sym(0);
+		L.seq.rep1 = zds_sym(1);
+		L.seq.rep2 = zds_sym(2);
+		L.seq.left = 0;
+		L.book.pos = L.book.lit_used = 0;
+		L.book.reach = 0;
+		L.book.sym = 0;
 		L.ll_log = L.ml_log = L.of_log = 0;
 		L.flags = 0;
-		L.nseq = L.left = 0;
+		L.nseq = 0;
 		L.status = ZS_OK;
-		L.rep0 = zds_sym(0);
-		L.rep1 = zds_sym(1);
-		L.rep2 = zds_sym(2);
-		L.pos = L.lit_used = 0;
-		L.reach = 0;
-		L.sym = 0;
 		u32 regen = 0;
 		if (mine && type != 2) regen = bsize;                       // Raw / RLE block
 		if (mine && type == 2 && (B.info & ZDS_I_BAD)) L.status = ZS_E_CORRUPT;
@@ -520,22 +390,28 @@ k_zds_entropy(ZdsJob J, u32* tabs, u32* queue, u32 want) {
 			const u8* fsrc = J.archive + J.off[U.k];
 			const u8* body = fsrc + U.ip + 3;
 			u32 n = U.hdr >> 3;
-			ZdsSect S;
-			zds_sections(body, n, S);  // validated by k_zds_modes
+			ZdSect S;
+			zd_sections(body, n, ZDS_MAXSEQ, S);  // validated by k_zds_modes
 			u32 st = ZS_OK;
 			// literals (Raw and RLE literals are read in place by the executor)
 			if (S.h.ltype >= 2) {
-				const u8* tsrc = nullptr;
-				u32 tn = 0;
-				if (S.h.ltype == 3 && U.src[0] != ZDS_NONE) {
-					ZdsBlk T = J.blk[U.src[0]];
-					tsrc = fsrc + T.ip + 3;
-					tn = T.hdr >> 3;
+				const u8* lp = body + S.h.hdr;
+				const u8* tree = lp;
+				u32 tn = S.h.comp;
+				if (S.h.ltype == 3) {  // Treeless: the tree of the block that last defined one (a block k_zds_modes validated)
+					tree = nullptr;
+					if (U.src[0] != ZDS_NONE) {
+						ZdsBlk T = J.blk[U.src[0]];
+						ZdLitHdr th;
+						zd_lit_header(fsrc + T.ip + 3, T.hdr >> 3, th);
+						tree = fsrc + T.ip + 3 + th.hdr;
+						tn = th.comp;
+					}
 				}
-				st = zds_literals(W, body, S.h, tsrc, tn, J.lit_stage + J.lit_off[itf]);
+				st = tree ? zd_warp_huf_literals(W, tree, tn, lp, S.h, J.lit_stage + J.lit_off[itf]) : ZS_E_CORRUPT;
 			}
 			ZdsLane V = L;  // (uniform copy of the fields the set-up writes; lane f keeps it)
-			V.nseq = V.left = S.nseq;
+			V.nseq = V.seq.left = S.nseq;
 			if (st == ZS_OK && S.nseq) {
 				const u8* p = S.tables;
 				const u8* end = body + n;
@@ -562,19 +438,12 @@ k_zds_entropy(ZdsJob J, u32* tabs, u32* queue, u32 want) {
 					V.of_log = logs[1];
 					V.ml_log = logs[2];
 					V.flags = fl;
-					ok = zs_back_init(V.b, p, (u32)(end - p));
-					if (ok) {
-						zs_back_reload(V.b);
-						V.sl = zs_back_read(V.b, V.ll_log);
-						V.so = zs_back_read(V.b, V.of_log);
-						V.sm = zs_back_read(V.b, V.ml_log);
-						ok = !zs_back_overflow(V.b);
-					}
+					ok = zd_seq_start(V.seq, p, end, V.ll_log, V.of_log, V.ml_log);
 				}
 				if (!ok) st = ZS_E_CORRUPT;
 			}
 			V.status = st;
-			if (st != ZS_OK) V.nseq = V.left = 0;
+			if (st != ZS_OK) V.nseq = V.seq.left = 0;
 			if (lane == (u32)f) L = V;
 			__syncwarp();
 		}
@@ -585,11 +454,11 @@ k_zds_entropy(ZdsJob J, u32* tabs, u32* queue, u32 want) {
 			const u32* oft = (L.flags & ZD_F_OF_DEF) ? ZS_OF_DEFAULT_DTABLE : my_slot + 1024;
 			u64* dst = J.seq_stage + (mine ? J.seq_off[i] : 0);
 			for (;;) {
-				u32 cnt = zg_min<u32>(64u, L.left);
+				u32 cnt = zg_min<u32>(64u, L.seq.left);
 				if (!__any_sync(ZG_FULL, cnt > 0)) break;
-				if (cnt && !zds_lane_decode(L, cnt, llt, mlt, oft, dst + (L.nseq - L.left))) {
+				if (cnt && !zd_lane_decode(L.seq, L.book, cnt, llt, mlt, oft, dst + (L.nseq - L.seq.left))) {
 					L.status = ZS_E_CORRUPT;
-					L.left = 0;
+					L.seq.left = 0;
 				}
 			}
 		}
@@ -597,21 +466,21 @@ k_zds_entropy(ZdsJob J, u32* tabs, u32* queue, u32 want) {
 		if (mine) {
 			if (type == 2 && L.status == ZS_OK) {
 				// all literals are emitted: those between the matches and the rest after the last sequence
-				if (L.lit_used > B.lit_regen) L.status = ZS_E_CORRUPT;
+				if (L.book.lit_used > B.lit_regen) L.status = ZS_E_CORRUPT;
 				else {
-					regen = L.pos + (B.lit_regen - L.lit_used);
+					regen = L.book.pos + (B.lit_regen - L.book.lit_used);
 					if (regen > ZS_BLOCK_MAX) L.status = ZS_E_CORRUPT;
 				}
 			}
 			ZdsRes R;
 			R.status = L.status;
 			R.regen = L.status == ZS_OK ? regen : 0;
-			R.rep[0] = L.rep0;
-			R.rep[1] = L.rep1;
-			R.rep[2] = L.rep2;
-			R.need_back = L.reach > 0 ? (u32)L.reach : 0u;
-			R.flags = L.sym ? ZDS_R_SYM : 0u;
-			R.lit_used = L.lit_used;
+			R.rep[0] = L.seq.rep0;
+			R.rep[1] = L.seq.rep1;
+			R.rep[2] = L.seq.rep2;
+			R.need_back = L.book.reach > 0 ? (u32)L.book.reach : 0u;
+			R.flags = L.book.sym ? ZDS_R_SYM : 0u;
+			R.lit_used = L.book.lit_used;
 			J.res[g] = R;
 		}
 		__syncwarp();
