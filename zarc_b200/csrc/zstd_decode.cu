@@ -152,6 +152,7 @@ k_zd_huf_literals(const u8* __restrict__ archive, const u64* __restrict__ sec_at
 			u32 mine = lane >= r0 && streams ? (1u << bits) | streams << 20 : 0;
 			u32 incl = zg_warp_incl_scan(mine);
 			u32 r1 = r0 + (u32)__popc(__ballot_sync(ZG_FULL, lane >= r0 && lane < ng && (incl & 0xfffffu) <= ZD_HL_TAB && (incl >> 20) <= 32));
+			ZD_SCHED_COUNT(1);
 			bool in = lane >= r0 && lane < r1 && streams;
 			u32 toff = (incl & 0xfffffu) - (mine & 0xfffffu), pre = (incl >> 20) - streams;
 			// 2. tables
@@ -335,6 +336,17 @@ k_zstd_decode_frames(const u8* __restrict__ archive, u64 archive_len, const u64*
 		__syncwarp();
 	}
 }
+
+#ifdef ZG_EMU
+u64 g_zd_sched[2];
+// the scheduling counters (ZD_SCHED_COUNT) since the last call, then zero
+extern "C" void zg_internal_sched_stats(u64 out[2]) {
+	for (int i = 0; i < 2; i++) {
+		out[i] = g_zd_sched[i];
+		g_zd_sched[i] = 0;
+	}
+}
+#endif
 
 // hand-out tuning (see the kernel): a batch holds at most 1/cap_div of a warp's fair share of the input but at least
 // min_batch bytes; frames so small that 32 of them stay below floor_bytes always go out as full rows

@@ -685,6 +685,15 @@ ZG_DEV_NOINLINE u32 zd_literals(ZdWarp* W, u32& flags, const u8* src, const ZdLi
 // ZD_DEFER = the sequence arena is full (nothing consumed), else a ZS_E_* code + 1.
 #define ZD_DEFER 1u
 #define ZD_ERR(c) ((c) + 1u)
+// The emulator build counts scheduling events no output shows, so that its tests can prove which ones a batch reached:
+// [0] block set-ups deferred for arena space, [1] rounds of the Huffman literals pre-pass (zg_internal_sched_stats).
+// The product build has no counter.
+#ifdef ZG_EMU
+extern u64 g_zd_sched[2];
+#define ZD_SCHED_COUNT(i) (zg_lane() == 0 ? (void)g_zd_sched[i]++ : (void)0)
+#else
+#define ZD_SCHED_COUNT(i) ((void)0)
+#endif
 ZG_DEV u32 zd_block_setup(ZdWarp* W, ZdLane& U, const u8* src, u32 n, u32* slot, u32& arena_used, u8* litbuf, ZdHufSave* save) {
 	ZdSect S;
 	// (the arena bounds the count: > 131072 sequences cannot come from a 128 KiB block)
@@ -706,7 +715,10 @@ ZG_DEV u32 zd_block_setup(ZdWarp* W, ZdLane& U, const u8* src, u32 n, u32* slot,
 		__syncwarp();
 		return 0;
 	}
-	if (arena_used + S.nseq > ZD_SEQ_ARENA) return ZD_DEFER;  // (an empty arena always fits a block)
+	if (arena_used + S.nseq > ZD_SEQ_ARENA) {  // (an empty arena always fits a block)
+		ZD_SCHED_COUNT(0);
+		return ZD_DEFER;
+	}
 	const u8* end = src + n;
 	const u8* p = S.tables;
 	u32 modes = S.modes;
