@@ -58,6 +58,15 @@ void zg_free_pinned(void* p);
 
 /* ---- parameters (libzstd's ZSTD_cParameter numbers; crates/zarc/src/encode.rs:12,84-89;
  *      CLI mapping crates/zarc-cli/src/pack.rs:89-114,140-195,227-237) ---------------------- */
+/* ZG_c_compressionLevel: -131072 .. 22 (0 = 3).  A negative level is libzstd's "fast" strategy with an acceleration
+ * of -level: every literals section is Raw (no Huffman), and from -2 down the match finder probes pairs of positions
+ * -level + 1 bytes apart (more after long stretches without a match).  The lower the level, the larger the frames.
+ * Speed does not fall in step: measured on a B200, -1 packs faster than level 1 (no Huffman step), -2 to -4 are no
+ * faster than -1 and can be slower than level 1 (the sampled parse advances less per step of the match finder), and
+ * from about -5 down the sampling makes packing faster again (see profiles/fast_levels_1gpu.json).  An explicit
+ * ZG_c_strategy >= 2 or ZG_c_searchLog overrides fast mode, as in libzstd: the level then acts as level 1.
+ * ZG_c_hashLog, ZG_c_minMatch and ZG_c_windowLog keep their meaning at negative levels.  Setting a negative level
+ * returns 0. */
 typedef enum {
 	ZG_c_compressionLevel = 100,
 	ZG_c_windowLog = 101,
@@ -87,7 +96,7 @@ void zg_hasher_free(zg_hasher*);
 typedef struct zg_cctx zg_cctx;
 zg_cctx* zg_cctx_create(void);                                 /* CCtx::try_create, NULL on failure */
 void zg_cctx_free(zg_cctx*);
-size_t zg_cctx_init(zg_cctx*, int level);                       /* CCtx::init(level); 0 => default 3 */
+size_t zg_cctx_init(zg_cctx*, int level);                       /* CCtx::init(level); 0 => default 3; < 0: fast, see above */
 size_t zg_cctx_set_parameter(zg_cctx*, int param, int value);   /* returns the value set, like libzstd */
 size_t zg_cctx_reset(zg_cctx*, int directive);                  /* CCtx::reset */
 size_t zg_cctx_set_stream(zg_cctx*, void* cuda_stream);         /* run on a caller-owned cudaStream_t */

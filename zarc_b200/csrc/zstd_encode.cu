@@ -892,7 +892,10 @@ struct ZeParams {
 	u32 min_match;  // shortest match emitted (4..7); minMatch
 	u32 max_dist;   // largest offset searched (<= 65535: matches never leave the 64 KiB the 16-bit table reaches); windowLog
 	u32 hlog_cap;   // hash table log2 (8..12); hashLog
+	u32 accel;      // negative levels: -level (1..ZE_ACCEL_MAX); 0 otherwise.  >= 2: strided fast parse (ze_fast_block)
+	u32 raw_lit;    // 1: every literals section Raw (negative levels, libzstd's literal compression off)
 };
+#define ZE_ACCEL_MAX 131072u  // -(the lowest level): the first step is already larger than a block
 
 // 16 bytes at an arbitrary address as four words.  Only aligned words are touched, and words that
 // start at or beyond `lim` read as zero (nothing past the block is dereferenced).
@@ -954,6 +957,29 @@ ZG_DEV void ze_try_candidate(const u8* src, const u8* lim, u32 n, u32 pos, i32 c
 		mlen = l;
 		moff = pos - (u32)cand;
 		bmatch = cand >= 4 ? (u32)__clz((int)(own_before ^ cand_before)) >> 3 : 0u;
+	}
+}
+
+// A match of L bytes at p (offset O) that the lane-capped extension stopped at ZE_LANE_CAP: the whole warp extends it,
+// 128 bytes per step.  Returns the full length.  All lanes call.
+ZG_DEV u32 ze_extend_warp(const u8* src, u32 n, u32 p, u32 L, u32 O) {
+	u32 lane = zg_lane();
+	for (;;) {
+		u32 q = p + L + 4 * lane;
+		u32 eq = 0;
+		if (q + 4 <= n) {
+			u32 x = zg_ld32(src + q) ^ zg_ld32(src + q - O);
+			eq = x ? (((u32)__ffs((int)x) - 1) >> 3) : 4;
+		} else {
+			while (q + eq < n && eq < 4 && src[q + eq] == src[q + eq - O]) eq++;
+		}
+		u32 full = __ballot_sync(ZG_FULL, eq == 4);
+		if (full == ZG_FULL) {
+			L += 128;
+			continue;
+		}
+		u32 first = (u32)__ffs((int)~full) - 1;
+		return L + 4 * first + __shfl_sync(ZG_FULL, eq, (int)first);
 	}
 }
 
@@ -1089,25 +1115,7 @@ ZG_DEV u32 ze_match_block(ZeMatchWarp* W, u64* seq, u8* lit, const u8* src, u32 
 			u32 L = __shfl_sync(ZG_FULL, mlen, (int)i), O = __shfl_sync(ZG_FULL, moff, (int)i);
 			u32 p = ip + i;
 			if (L >= ZE_LANE_CAP && p + L < n) {
-				// whole-warp extension, 128 bytes per step
-				for (;;) {
-					u32 q = p + L + 4 * lane;
-					u32 eq = 0;
-					if (q + 4 <= n) {
-						u32 x = zg_ld32(src + q) ^ zg_ld32(src + q - O);
-						eq = x ? (((u32)__ffs((int)x) - 1) >> 3) : 4;
-					} else {
-						while (q + eq < n && eq < 4 && src[q + eq] == src[q + eq - O]) eq++;
-					}
-					u32 full = __ballot_sync(ZG_FULL, eq == 4);
-					if (full == ZG_FULL) {
-						L += 128;
-						continue;
-					}
-					u32 first = (u32)__ffs((int)~full) - 1;
-					L += 4 * first + __shfl_sync(ZG_FULL, eq, (int)first);
-					break;
-				}
+				L = ze_extend_warp(src, n, p, L, O);
 				if (lane == i) mlen = L;
 			}
 			cur = p + L;
@@ -1141,6 +1149,118 @@ ZG_DEV u32 ze_match_block(ZeMatchWarp* W, u64* seq, u8* lit, const u8* src, u32 
 		for (u32 k = lane; k < rest; k += 32) lit[lpos + k] = src[start + k];
 		lpos += rest;
 	}
+	__syncwarp();
+	*lit_count = lpos;
+	return nseq;
+}
+
+// Levels -2 and below: libzstd's fast-strategy stepping (ZSTD_compressBlock_fast, targetLength = prm.accel) restated
+// for a warp.  Positions are probed in pairs (q, q + 1) whose starts are `step` apart: step = accel + 1 right after a
+// match and one more for every ZE_STEP_INCR bytes parsed since.  A window is 16 pairs, lane 2k + j probing
+// p + k * step + j; only probed positions enter the table (same table, hash and distance limit as ze_match_block).  The
+// first probe with a match of min_match bytes or more is taken, extended forward (the lane, then the whole warp) and
+// backward as far as the end of the previous match -- a sampled parse lands inside most matches, and without the
+// catch-up their heads would stay literals -- then the first probe at or after its end, and so on.  The next window
+// starts at the last match's end (or after the window when there was none).  Same outputs as ze_match_block:
+// sequences with plain offsets, literals gathered into `lit`.
+#define ZE_STEP_INCR 128u
+ZG_DEV u32 ze_fast_block(ZeMatchWarp* W, u64* seq, u8* lit, const u8* src, u32 n, const ZeParams& prm, u32* lit_count) {
+	u32 lane = zg_lane();
+	u32 ltmask = zg_lanemask_lt();
+	const u32 minmatch = prm.min_match, maxdist = prm.max_dist;
+	u32 hlog = 8;
+	while (hlog < prm.hlog_cap && (1u << hlog) < n) hlog++;
+	u16* htab = W->htab;
+	const u8* lim = src + n;
+	{
+		u32* h32 = (u32*)htab;
+		for (u32 i = lane; i < zg_min<u32>(1u << hlog, ZE_TAB_ENTRIES) / 2; i += 32) h32[i] = 0;
+	}
+	__syncwarp();
+	u32 mend = 0;  // end of the last match = start of the pending literals
+	u32 lpos = 0, nseq = 0, ip = 0;
+	while (ip < n && nseq < ZE_MAXSEQ - 32) {
+		u32 step = prm.accel + 1 + (ip - mend) / ZE_STEP_INCR;  // (<= 2^17 + 2^10: the window's positions fit 32 bits)
+		u32 pos = ip + (lane >> 1) * step + (lane & 1);
+		bool valid = pos + 4 <= n;
+		u32 own[4] = {0, 0, 0, 0};
+		if (valid) ze_ld128(src + pos, lim, own);
+		u32 v = own[0];
+		u32 h = valid ? ze_hash4(v, hlog) : (0x80000000u | lane);
+		u32 te = valid ? htab[h] : 0;
+		u32 peers = __match_any_sync(ZG_FULL, h);
+		// candidate: nearest earlier lane with the same hash, else the table entry
+		u32 lower = peers & ltmask;
+		u32 lower_pos = __shfl_sync(ZG_FULL, pos, lower ? (int)(31u - (u32)__clz((int)lower)) : (int)lane);
+		i32 cand = -1;
+		if (valid) {
+			if (lower) {
+				cand = (i32)lower_pos;
+			} else {
+				i32 c = (i32)((pos & ~0xffffu) | te);
+				if (c >= (i32)pos) c -= 65536;
+				cand = c;
+			}
+			if (cand >= 0 && pos - (u32)cand > maxdist) cand = -1;
+		}
+		u32 mlen = 0;
+		if (cand >= 0) {
+			u32 c[4];
+			ze_ld128(src + cand, lim, c);
+			if (c[0] == v) {
+				u32 maxl = zg_min<u32>(n - pos, ZE_LANE_CAP);
+				mlen = ze_eq16(own, c);
+				while (mlen < maxl && (mlen & 15u) == 0) {
+					u32 a[4];
+					ze_ld128(src + pos + mlen, lim, a);
+					ze_ld128(src + (u32)cand + mlen, lim, c);
+					u32 e = ze_eq16(a, c);
+					mlen += e;
+					if (e < 16) break;
+				}
+				mlen = zg_min<u32>(mlen, maxl);
+			}
+		}
+		// greedy in position order: the first probe with a match, then the first one at or after its end, and so on
+		u32 has = __ballot_sync(ZG_FULL, mlen >= minmatch);
+		u32 next = ip + 16 * step;  // where the next window starts: here, or the last match's end
+		while (has) {
+			u32 i = (u32)__ffs((int)has) - 1u;
+			u32 L = __shfl_sync(ZG_FULL, mlen, (int)i), q = __shfl_sync(ZG_FULL, pos, (int)i);
+			u32 O = q - (u32)__shfl_sync(ZG_FULL, cand, (int)i);
+			if (L >= ZE_LANE_CAP && q + L < n) L = ze_extend_warp(src, n, q, L, O);
+			// backward, 32 bytes per step: never before the previous match's end nor before the block
+			u32 back = 0;
+			for (;;) {
+				u32 k = back + lane + 1;
+				bool eq = k <= q - mend && k <= q - O && src[q - k] == src[q - O - k];
+				u32 all = __ballot_sync(ZG_FULL, eq);
+				if (all == ZG_FULL) {
+					back += 32;
+					continue;
+				}
+				back += (u32)__ffs((int)~all) - 1u;
+				break;
+			}
+			u32 ll = q - back - mend;
+			for (u32 k = lane; k < ll; k += 32) lit[lpos + k] = src[mend + k];
+			if (lane == 0) seq[nseq] = ZE_SEQ_PACK(O, ll, L + back);
+			lpos += ll;
+			nseq++;
+			mend = q + L;
+			next = mend;
+			has &= __ballot_sync(ZG_FULL, pos >= mend);
+		}
+		// After a match the next window starts at its end with the first step again, as libzstd's parse does.  The probes
+		// of this window at or after that point are probed again there, so they stay out of the table (a probe would find
+		// itself); the others enter it, the highest lane of each hash group.
+		u32 ins = __ballot_sync(ZG_FULL, valid && pos < next);
+		if (((ins >> lane) & 1u) && ((peers & ins) >> lane) == 1u) htab[h] = (u16)pos;
+		__syncwarp();
+		ip = next;
+	}
+	for (u32 k = lane; k < n - mend; k += 32) lit[lpos + k] = src[mend + k];
+	lpos += n - mend;
 	__syncwarp();
 	*lit_count = lpos;
 	return nseq;
@@ -1235,6 +1355,35 @@ ZG_DEV bool ze_assign_repcodes(ZeMatchWarp* W, u64* seq, u32 nseq, bool first_bl
 }
 
 // ---------------------------------------------------------------------------------------------
+// A Raw (mode 0) or RLE (mode 1) literals section at p: a header of 1, 2 or 3 bytes (Size_Format by nlit, RFC 8878
+// §3.1.1.3.1.1) and the payload.  Returns its end, or null when it does not fit before `end`.  All lanes call.
+ZG_DEV u8* ze_literals_plain(const u8* lit, u32 nlit, u32 mode, u8* p, u8* end) {
+	u32 lane = zg_lane();
+	u32 payload = mode == 1 ? 1 : nlit;
+	u32 hdr = nlit < 32 ? 1 : nlit < 4096 ? 2 : 3;
+	if (p + hdr + payload > end) return nullptr;
+	if (lane == 0) {
+		if (hdr == 1) p[0] = (u8)(mode | (nlit << 3));
+		else if (hdr == 2) {
+			u32 v = mode | (1u << 2) | (nlit << 4);
+			p[0] = (u8)v;
+			p[1] = (u8)(v >> 8);
+		} else {
+			u32 v = mode | (3u << 2) | (nlit << 4);
+			p[0] = (u8)v;
+			p[1] = (u8)(v >> 8);
+			p[2] = (u8)(v >> 16);
+		}
+	}
+	p += hdr;
+	if (mode == 1) {
+		if (lane == 0) p[0] = lit[0];
+	} else {
+		for (u32 i = lane; i < nlit; i += 32) p[i] = lit[i];
+	}
+	return p + payload;
+}
+
 // K3a: the literals section of one block into dst[0..cap).  Returns its size, or 0 if the block
 // cannot end up smaller than raw.  All lanes call.
 ZG_DEV u32 ze_literals_section(ZeWarp* W, const u8* lit, u32 nlit, u8* dst, u32 cap) {
@@ -1341,33 +1490,20 @@ ZG_DEV u32 ze_literals_section(ZeWarp* W, const u8* lit, u32 nlit, u8* dst, u32 
 			}
 		}
 	} else {
-		u32 payload = mode == 1 ? 1 : nlit;
-		u32 hdr = nlit < 32 ? 1 : nlit < 4096 ? 2 : 3;
-		if (p + hdr + payload > end) return 0;
-		if (lane == 0) {
-			if (hdr == 1) p[0] = (u8)(mode | (nlit << 3));
-			else if (hdr == 2) {
-				u32 v = mode | (1u << 2) | (nlit << 4);
-				p[0] = (u8)v;
-				p[1] = (u8)(v >> 8);
-			} else {
-				u32 v = mode | (3u << 2) | (nlit << 4);
-				p[0] = (u8)v;
-				p[1] = (u8)(v >> 8);
-				p[2] = (u8)(v >> 16);
-			}
-		}
-		p += hdr;
-		if (mode == 1) {
-			if (lane == 0) p[0] = lit[0];
-		} else {
-			for (u32 i = lane; i < nlit; i += 32) p[i] = lit[i];
-		}
-		p += payload;
+		p = ze_literals_plain(lit, nlit, mode, p, end);
+		if (!p) return 0;
 	}
 	__syncwarp();
 	__syncwarp();
 	return (u32)(p - dst);
+}
+
+// K3a of the negative levels: a Raw literals section, the header and a copy.  Same contract as ze_literals_section.
+ZG_DEV u32 ze_literals_raw(const u8* lit, u32 nlit, u8* dst, u32 cap) {
+	if (cap < 16) return 0;
+	u8* p = ze_literals_plain(lit, nlit, 0, dst, dst + cap);
+	__syncwarp();
+	return p ? (u32)(p - dst) : 0u;
 }
 
 // K3b1: sequence codes + histograms, table modes, table descriptions into dst[0..cap) (dst = just
@@ -1745,7 +1881,7 @@ __global__ void __launch_bounds__(256) k_ze_order_scatter(ZeJob J, u32 nchunks, 
 	order[atomicAdd(&bins[ze_obin_slot(J, B, nchunks)], 1u)] = (u32)b;
 }
 
-// K2
+// K2.  WAYS = 0: the strided fast parse of levels -2 and below
 template <int WAYS>
 __global__ void __launch_bounds__(ZE_WARPS * 32, ZE_MIN_CTAS) k_zstd_match_blocks(ZeJob J, u32 chunk, u32* queue, ZeParams prm) {
 	ZG_DYN_SMEM(ZeMatchWarp, sm);
@@ -1759,7 +1895,9 @@ __global__ void __launch_bounds__(ZE_WARPS * 32, ZE_MIN_CTAS) k_zstd_match_block
 		u8* lit = J.litbuf + rel;
 		u32 nseq = ZE_RAW, nlit = 0;
 		if (B.n >= 16) {
-			nseq = ze_match_block<WAYS>(W, seq, lit, J.blob + J.file_off[B.f] + B.j * ZS_BLOCK_MAX, B.n, prm, &nlit);
+			const u8* src = J.blob + J.file_off[B.f] + B.j * ZS_BLOCK_MAX;
+			if constexpr (WAYS == 0) nseq = ze_fast_block(W, seq, lit, src, B.n, prm, &nlit);
+			else nseq = ze_match_block<WAYS>(W, seq, lit, src, B.n, prm, &nlit);
 			__syncwarp();
 			// later blocks of a frame are encoded independently of their predecessors: unknown history
 			if (!ze_assign_repcodes(W, seq, nseq, B.j == 0)) nseq = ZE_RAW;
@@ -1772,8 +1910,8 @@ __global__ void __launch_bounds__(ZE_WARPS * 32, ZE_MIN_CTAS) k_zstd_match_block
 	}
 }
 
-// K3a
-__global__ void __launch_bounds__(ZE_WARPS * 32, ZE_ENT_CTAS) k_zstd_literals(ZeJob J, u32 chunk, u32* queue) {
+// K3a.  raw_lit: Raw sections only (negative levels): no histogram, no Huffman
+__global__ void __launch_bounds__(ZE_WARPS * 32, ZE_ENT_CTAS) k_zstd_literals(ZeJob J, u32 chunk, u32* queue, u32 raw_lit) {
 	ZG_DYN_SMEM(ZeWarp, sm);
 	ZeWarp* W = &sm[threadIdx.x >> 5];
 	u32 lane = threadIdx.x & 31;
@@ -1784,7 +1922,8 @@ __global__ void __launch_bounds__(ZE_WARPS * 32, ZE_ENT_CTAS) k_zstd_literals(Ze
 		if (m.nseq != ZE_RAW) {
 			ZeBlk B = ze_block(J, b);
 			u64 rel = B.soff - (u64)chunk * J.chunk_bytes;
-			litsec = ze_literals_section(W, J.litbuf + rel, m.nlit, J.comp + B.soff, B.n - 1);
+			litsec = raw_lit ? ze_literals_raw(J.litbuf + rel, m.nlit, J.comp + B.soff, B.n - 1)
+			                 : ze_literals_section(W, J.litbuf + rel, m.nlit, J.comp + B.soff, B.n - 1);
 		}
 		__syncwarp();
 		if (lane == 0) J.meta[b].litsec = litsec;
@@ -1843,9 +1982,17 @@ extern "C" void zg_internal_set_encode_chunk_bytes(u64 v) { g_ze_chunk_bytes = v
 //   hashLog    table of 2^clamp(hashLog, 8, 12) positions             minMatch   4..7 (3 is refused by zg_cctx_set_parameter)
 //   windowLog  matches no further back than min(2^windowLog, 65535)
 // chainLog and targetLength have no counterpart here and are refused when set (zg_cctx_set_parameter).
+// A negative level is libzstd's fast strategy with targetLength = -level, which also turns literal compression off:
+// Raw literals, and from -2 down the strided parse of ze_fast_block (level -1 keeps level 1's greedy parse: libzstd
+// steps only from targetLength 2).  An explicit strategy >= 2 or searchLog asks for another strategy than fast, and
+// then a negative level resolves as level 1 does.
 static ZeParams ze_resolve_params(const ZgCParams& cp) {
 	ZeParams p;
 	int level = cp.level;
+	const bool fast = level < 0 && cp.strategy < 2 && cp.search_log == 0;
+	p.accel = fast ? (u32)zg_min<int>(-level, (int)ZE_ACCEL_MAX) : 0u;
+	p.raw_lit = fast ? 1u : 0u;
+	if (level < 0) level = 1;
 	p.lazy = level >= 3 ? 1 : 0;
 	p.ways = level >= 9 ? 4 : level >= 6 ? 2 : 1;
 	if (cp.strategy > 0) {
@@ -1905,7 +2052,8 @@ size_t zg_zstd_encode_run(cudaStream_t s, ZgZeWork& w, const u8* blob, const u64
 	static ZgPerDevice attr_dev;
 	bool& attr_set = *attr_dev.slot();
 	if (!attr_set) {
-		if (cudaFuncSetAttribute(k_zstd_match_blocks<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_m) != cudaSuccess ||
+		if (cudaFuncSetAttribute(k_zstd_match_blocks<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_m) != cudaSuccess ||
+		    cudaFuncSetAttribute(k_zstd_match_blocks<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_m) != cudaSuccess ||
 		    cudaFuncSetAttribute(k_zstd_match_blocks<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_m) != cudaSuccess ||
 		    cudaFuncSetAttribute(k_zstd_match_blocks<4>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_m) != cudaSuccess ||
 		    cudaFuncSetAttribute(k_zstd_literals, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_l) != cudaSuccess ||
@@ -1930,12 +2078,13 @@ size_t zg_zstd_encode_run(cudaStream_t s, ZgZeWork& w, const u8* blob, const u64
 	for (u32 k = 0; k < nchunks; k++) {
 		u32* qk = q + (size_t)k * ZE_NQ;
 		zg_prof_begin(ZG_K_MATCH, s);
-		if (prm.ways == 4) ZG_LAUNCH(k_zstd_match_blocks<4>, grid_m, ZE_WARPS * 32, smem_m, s, J, k, qk + 0, prm);
+		if (prm.accel >= 2) ZG_LAUNCH(k_zstd_match_blocks<0>, grid_m, ZE_WARPS * 32, smem_m, s, J, k, qk + 0, prm);
+		else if (prm.ways == 4) ZG_LAUNCH(k_zstd_match_blocks<4>, grid_m, ZE_WARPS * 32, smem_m, s, J, k, qk + 0, prm);
 		else if (prm.ways == 2) ZG_LAUNCH(k_zstd_match_blocks<2>, grid_m, ZE_WARPS * 32, smem_m, s, J, k, qk + 0, prm);
 		else ZG_LAUNCH(k_zstd_match_blocks<1>, grid_m, ZE_WARPS * 32, smem_m, s, J, k, qk + 0, prm);
 		zg_prof_end(ZG_K_MATCH, s);
 		zg_prof_begin(ZG_K_LITERALS, s);
-		ZG_LAUNCH(k_zstd_literals, grid_e, ZE_WARPS * 32, smem_l, s, J, k, qk + 1);
+		ZG_LAUNCH(k_zstd_literals, grid_e, ZE_WARPS * 32, smem_l, s, J, k, qk + 1, prm.raw_lit);
 		zg_prof_end(ZG_K_LITERALS, s);
 		zg_prof_begin(ZG_K_SEQUENCES, s);
 		ZG_LAUNCH(k_zstd_sequences, grid_e, ZE_WARPS * 32, smem_q, s, J, k, qk + 2);

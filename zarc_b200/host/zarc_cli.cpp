@@ -45,7 +45,9 @@ static const uint64_t BATCH_BYTES = getenv("ZARC_BATCH_MB") ? (uint64_t)atoll(ge
 	        "zarc-b200 -- zarc archives with the content path on the GPU\n\n"
 	        "  zarc-b200 pack --output <PATH> [--level <N>] [--zstd <name=value>]... [-L|--follow-symlinks] <PATHS>...\n"
 	        "  zarc-b200 unpack [--filter <REGEX>]... [--verify <DIGEST>] <PATH>\n"
-	        "  zarc-b200 list-files [--only-files] [--decorate] [--filter <REGEX>]... <PATH>\n");
+	        "  zarc-b200 list-files [--only-files] [--decorate] [--filter <REGEX>]... <PATH>\n\n"
+	        "  --level: -131072 to 22 (default 3).  Negative levels store literals uncompressed and sample the input:\n"
+	        "           larger archives; -1 packs faster than 1, -2 to -4 are no faster than -1, -5 and below faster again\n");
 	exit(code);
 }
 
